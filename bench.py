@@ -4,11 +4,15 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: the reference's CPU algorithm on host cores
+    python bench.py --gpus 1 --steps K --dump-outputs DIR    # also write the last timed step's result to DIR/*.npy
 
 One step = one ELBO+gradient evaluation over one minibatch of N_b points per GPU (weak scaling: every rank owns N_b
 points x S samples) followed, for N > 1, by ONE NCCL sum-allreduce of the flat [ELBO terms, gradients] buffer.
 `value` times device-resident inputs; `e2e` times the host-buffer entry point (H2D of the minibatch, D2H of the result).
 Prints ONE JSON line on rank 0.
+
+The inputs (parameters, minibatches, Philox seeds) depend only on the arguments, so two builds run with the same arguments
+can be compared output for output through --dump-outputs.
 """
 import argparse
 import json
@@ -25,6 +29,44 @@ if ROOT not in sys.path:
 METRIC = "DGP ELBO+grad point-samples/s"
 UNIT = "point-samples/s"
 FP64_PEAK_FALLBACK_TFLOPS = 37.07   # profiles/r0*_fp64_peaks.json (DMMA.8x8x4 register-resident loop, this pool's B200)
+DUMP_LIMIT_BYTES = 64 << 20
+N_POOL = 4   # distinct minibatches cycled through (fresh X, Y every step)
+
+
+def step_inputs(i, nb, world=1, rank=0):
+    """Inputs of timed step i on `rank` besides the model: the synthetic.minibatch index of its nb points (pool entry
+    i % N_POOL), the global index of its first point (Philox counters), the ELBO scale (N = 1M points behind the
+    minibatch, BASELINE config 2) and the Philox seed."""
+    return {"batch": (i % N_POOL) * world + rank, "n_offset": (i * world + rank) * nb, "scale": 1.0e6 / (nb * world),
+            "seed": 1234 + i}
+
+
+def step_outputs(model, flat):
+    """The flat [data term, KL, gradients] buffer of one step as named float64 arrays, gradients named like
+    DGP_Base.ELBO_and_grads."""
+    flat = flat.detach().cpu()
+    names = {model.likelihood.likelihood.variance: "grad_lik_var"}
+    for i, l in enumerate(model.layers):
+        for key, p in (("Z", l.feature.Z), ("lengthscales", l.kern.lengthscales), ("variance", l.kern.variance),
+                       ("q_mu", l.q_mu), ("q_sqrt", l.q_sqrt)):
+            names[p] = f"grad_layers.{i}.{key}"
+    out = {"data_term": flat[0], "kl": flat[1], "elbo": flat[0] - flat[1]}
+    out.update({names[p]: g for p, g in model.unpack_grads(flat).items()})
+    return {k: v.numpy().astype("float64") for k, v in out.items()}
+
+
+def dump_outputs(directory, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes every array as directory/<name>.npy in float64. When they add up to more than `limit` bytes, an array larger
+    than an equal share of the limit is replaced by a fixed, seeded sample of its flattened entries (sorted positions), the
+    same positions for the same shapes on every run."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    cap = None if sum(a.size for a in arrays.values()) * 8 <= limit else limit // 8 // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if cap is not None and a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def load_synthetic(package):
@@ -344,7 +386,13 @@ def main():
     ap.add_argument("--nb-cpu", type=int, default=512, help="points of the bounded CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip extra.configs (configs 3 and 5) and extra.strong_scaling")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the ELBO terms and gradients of the last timed step (rank 0) "
+                    "as DIR/<name>.npy, float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     synthetic = load_synthetic(package=args.impl == "ours")
@@ -390,13 +438,11 @@ def main():
     model = synthetic.model_from_problem(prob, cfg["S"])
     sharded = ShardedELBO(model)
     nb, S = args.nb, cfg["S"]
-    n_pool = 4   # distinct minibatches cycled through (fresh X, Y every step)
     pool_host = []
-    for i in range(n_pool):
-        X, Y = synthetic.minibatch(cfg["D0"], nb, i * world + rank)
+    for i in range(N_POOL):
+        X, Y = synthetic.minibatch(cfg["D0"], nb, step_inputs(i, nb, world, rank)["batch"])
         pool_host.append((torch.from_numpy(X).pin_memory(), torch.from_numpy(Y).pin_memory()))
     pool_dev = [(x.cuda(), y.cuda()) for x, y in pool_host]
-    scale = 1.0e6 / (nb * world)   # N = 1M points behind the minibatch (BASELINE config 2)
 
     def sync_all():
         torch.cuda.synchronize()
@@ -405,12 +451,14 @@ def main():
             torch.cuda.synchronize()
 
     def step_dev(i):
-        X, Y = pool_dev[i % n_pool]
-        return sharded.step(X, Y, n_offset=(i * world + rank) * nb, scale=scale, seed=1234 + i)
+        X, Y = pool_dev[i % N_POOL]
+        s = step_inputs(i, nb, world, rank)
+        return sharded.step(X, Y, n_offset=s["n_offset"], scale=s["scale"], seed=s["seed"])
 
     def step_host(i):
-        X, Y = pool_host[i % n_pool]
-        return sharded.step_host(X, Y, n_offset=(i * world + rank) * nb, scale=scale, seed=1234 + i)
+        X, Y = pool_host[i % N_POOL]
+        s = step_inputs(i, nb, world, rank)
+        return sharded.step_host(X, Y, n_offset=s["n_offset"], scale=s["scale"], seed=s["seed"])
 
     def timed(fn, k):
         import gc
@@ -462,7 +510,7 @@ def main():
         sscale = 1.0e6 / nb
 
         def step_strong(i):
-            X, Y = pool_dev[i % n_pool]
+            X, Y = pool_dev[i % N_POOL]
             return sharded.step(X[lo:hi], Y[lo:hi], n_offset=i * nb + lo, scale=sscale, seed=1234 + i)
         for i in range(warmup):
             step_strong(i)
@@ -476,6 +524,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, step_outputs(model, out))
 
     ps_per_step = nb * S * world
     ms_step = ms_total / args.steps
@@ -562,7 +612,7 @@ def main():
     if world == 1 and not args.no_extras:
         del pool_dev, sharded, model
         torch.cuda.empty_cache()
-        extra["configs"] = forward_extras(D, synthetic, torch, max(2, min(args.steps, 4)), peak, not args.no_cpu_baseline)
+        extra["configs"] = forward_extras(D, synthetic, torch, args.steps, peak, not args.no_cpu_baseline)
         extra["fp64_pipe"] = {"dmma_dfma_co_issue": False, "source": "profiles/r02_fp64_peaks.json (tools/fp64_peaks.cu: DMMA-only 37.1, "
                               "DFMA-only 36.5, both in one warp 35.8, warp-specialised 36.4 TFLOP/s: one shared FP64 pipe, so the DMMA "
                               "peak is the ceiling of the kernels' mixed DMMA + DFMA instruction stream)"}

@@ -1,7 +1,8 @@
-"""Runs the reference's OWN source (`/root/reference/dgp_dace`, imported unmodified) on the stand-in tensorflow / gpflow /
-tensorflow_probability modules of tests/ref_shim (torch-CPU float64). Test infrastructure: used by
-tests/test_reference_exec.py and tests/golden/make_golden.py in the build container; `/root/reference` does not exist on
-the GPU box, where only the committed vectors under tests/golden/ are used."""
+"""Runs the reference's OWN source (the `dgp_dace` package of a reference checkout whose root DGP_REFERENCE_ROOT names,
+imported unmodified) on the stand-in tensorflow / gpflow / tensorflow_probability modules of tests/ref_shim (torch-CPU
+float64). Test infrastructure: used by tests/test_reference_exec.py and the tests/golden/make_golden*.py scripts. The
+repository does not contain the reference; without a checkout the tests compare with the reference outputs stored under
+tests/golden/."""
 import importlib
 import os
 import sys
@@ -12,11 +13,11 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SHIM = os.path.join(HERE, "ref_shim")
-REFERENCE = os.environ.get("DGP_REFERENCE_ROOT", "/root/reference")
+REFERENCE = os.environ.get("DGP_REFERENCE_ROOT", "")
 
 
 def available():
-    return os.path.isdir(os.path.join(REFERENCE, "dgp_dace"))
+    return bool(REFERENCE) and os.path.isdir(os.path.join(REFERENCE, "dgp_dace"))
 
 
 _mods = None
@@ -28,7 +29,7 @@ def load():
     if _mods is not None:
         return _mods
     if not available():
-        raise RuntimeError("reference tree not found at " + REFERENCE)
+        raise RuntimeError("no reference checkout: set DGP_REFERENCE_ROOT to the directory that holds dgp_dace/")
     for p in (REFERENCE, SHIM):
         if p not in sys.path:
             sys.path.insert(0, p)

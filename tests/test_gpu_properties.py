@@ -392,3 +392,33 @@ def test_kernel_exponential_is_accurate_to_ulps():
         Km = cls(variance=1.0, lengthscales=1.0).K(x[1:], np.zeros((1, 1))).cpu().numpy()[:, 0]
         refm = f(x[1:, 0])
         assert (np.abs(Km - refm) / refm).max() < 1e-14
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs writes the ELBO terms and the gradients of its last timed step: the same arrays come out of
+    one direct elbo_flat call on that step's inputs (bench.step_inputs: minibatch, Philox seed, point offset and scale)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import bench
+    from dgp_toolbox_b200 import synthetic
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    steps, nb = bench.N_POOL + 2, 512      # the last step reuses a pool minibatch with its own seed and point offset
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                          "--nb", str(nb), "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps
+    model, cfg = _c2_model()
+    s = bench.step_inputs(steps - 1, nb)
+    X, Y = synthetic.minibatch(cfg["D0"], nb, s["batch"])
+    flat = model.elbo_flat((X, Y), scale=s["scale"], seed=s["seed"], n_offset=s["n_offset"])
+    ref = bench.step_outputs(model, flat)
+    assert sorted(os.listdir(tmp_path)) == sorted(k + ".npy" for k in ref)
+    for k, v in ref.items():
+        got = np.load(os.path.join(tmp_path, k + ".npy"))
+        assert got.dtype == np.float64 and got.shape == v.shape, k
+        assert np.max(np.abs(got - v), initial=0.0) <= 1e-11 * max(np.max(np.abs(v), initial=0.0), 1e-300), k
+    assert abs(float(np.load(os.path.join(tmp_path, "elbo.npy"))) - line["elbo_last_step"]) <= 1e-12 * abs(line["elbo_last_step"])

@@ -165,6 +165,22 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["e2e"]["h2d_bytes_per_step"] == 0 and d["value"] > 0
 
 
+def test_bench_dump_outputs_keep_to_the_size_limit(tmp_path):
+    """bench.py --dump-outputs: float64 arrays under the size limit are written whole; above it, the large arrays become the
+    same seeded sample of their entries on every run."""
+    import bench
+    arrays = {"small": np.arange(10.0), "large": np.random.default_rng(1).standard_normal((3, 100, 100))}
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    for k, v in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "whole" / (k + ".npy")), v)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, limit=1 << 12)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= (1 << 12) + 2 * 128   # + the .npy headers
+    small, large = np.load(tmp_path / "a" / "small.npy"), np.load(tmp_path / "a" / "large.npy")
+    assert np.array_equal(small, arrays["small"]) and large.dtype == np.float64 and large.shape == ((1 << 12) // 16,)
+    assert np.all(np.isin(large, arrays["large"])) and np.array_equal(large, np.load(tmp_path / "b" / "large.npy"))
+
+
 def test_chunked_oracle_equals_single_pass():
     """oracle.elbo_and_grads_chunked (used by the full-size GPU parity tests) == oracle.elbo_and_grads on the same Philox draws."""
     import torch
