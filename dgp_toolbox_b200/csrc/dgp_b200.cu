@@ -618,6 +618,13 @@ struct ChunkIO {   // caller-visible arrays [S][N][D_l], any may be null
 
 struct Temps { double *t0 = nullptr, *t1 = nullptr, *t2 = nullptr; };   // three [maxMp][Pp] planes
 
+// q_mu is staged whole in shared memory by the unfused moments kernel
+bool moments_fit(dgp_ctx* c, const LayerWs& w) {
+  if (w.fcfg >= 0 || (size_t)w.M * w.D_out * sizeof(double) <= 160 * 1024) return true;
+  c->err = "unfused conditional: M * D_out * 8 bytes of q_mu exceed the 160 KiB staged per CTA (fused path: M <= 256, D_out <= 16)";
+  return false;
+}
+
 int forward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, ChunkLayer& cl, const Temps& tmp, bool stash,
                   double* Tshared, int layer, long Nc, long S, long N_total, long n0, unsigned long long seed, long n_offset,
                   const ChunkIO& io, bool need_sample) {
@@ -692,10 +699,7 @@ int forward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, ChunkLa
   a.xFvar = (io.Fvars && io.Fvars[layer]) ? io.Fvars[layer] : nullptr;
   a.xF = (io.Fs && io.Fs[layer]) ? io.Fs[layer] : nullptr;
   const size_t smem = (size_t)w.M * D * sizeof(double);
-  if (smem > 160 * 1024) {   // q_mu is staged whole in shared memory by the unfused moments kernel
-    c->err = "unfused conditional: M * D_out * 8 bytes of q_mu exceed the 160 KiB staged per CTA (fused path: M <= 256, D_out <= 16)";
-    return DGP_ERR_UNSUPPORTED;
-  }
+  if (!moments_fit(c, w)) return DGP_ERR_UNSUPPORTED;
   return dispatch_dmax(D, [&](auto dm) -> int {
     constexpr int DM = decltype(dm)::value;
     if (!c->dry) {
@@ -805,16 +809,17 @@ int backward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const 
     r.W = Kbar; r.A = nullptr; r.gq = up.gq; r.Gbar = Gbar; r.Xin = cl.Xin; r.xmod = cl.xmod; r.Z = d.Z; r.ls = d.lengthscales;
     r.var = d.variance; r.M = w.M; r.Mp = Mp; r.D_in = w.D_in; r.P = P; r.Pp = Pp; r.Gm = up.Gm; r.D_out = D;
     r.mean_kind = d.mean_kind; r.mfW = d.mf_W; r.kind = d.kernel_kind; r.dXin = dXin; r.XaugPad = XaugPad; r.part = rbf_part;
-    const bool small = Pp / 128 < 2L * c->num_sms;   // latency-bound launch: 64-column blocks with 4 row groups
+    // latency-bound launch: 64-column blocks with 4 row groups, where their shared memory fits
+    const bool small = Pp / 128 < 2L * c->num_sms && rbf_bwd_smem_bytes(w.M, w.D_in) <= kRbfBwdSmemMax;
     nbv = small ? Pp / kRbfCols : Pp / 128;
     const size_t smemv = small ? rbf_bwd_smem_bytes(w.M, w.D_in) : ((size_t)w.M * w.D_in + kMaxD + 32) * sizeof(double);
     RC(dispatch_dmax(w.D_in, [&](auto dm) -> int {
       constexpr int DM = decltype(dm)::value;
       if (small) {
-        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
         LAUNCH((rbf_bwd2d_kernel<DM, true>), (unsigned)nbv, 256, smemv, r);
       } else {
-        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
         LAUNCH((rbf_bwd_kernel<DM, true>), (unsigned)nbv, 128, smemv, r);
       }
       return DGP_OK;
@@ -873,16 +878,17 @@ int backward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const 
   r.W = W; r.A = cl.A; r.gq = up.gq; r.Gbar = Gbar; r.Xin = cl.Xin; r.xmod = cl.xmod; r.Z = d.Z; r.ls = d.lengthscales;
   r.var = d.variance; r.M = w.M; r.Mp = Mp; r.D_in = w.D_in; r.P = P; r.Pp = Pp; r.Gm = up.Gm; r.D_out = D;
   r.mean_kind = d.mean_kind; r.mfW = d.mf_W; r.kind = d.kernel_kind; r.dXin = dXin; r.XaugPad = XaugPad; r.part = rbf_part;
-  const bool small = Pp / 128 < 2L * c->num_sms;   // latency-bound launch: 64-column blocks with 4 row groups
+  // latency-bound launch: 64-column blocks with 4 row groups, where their shared memory fits
+  const bool small = Pp / 128 < 2L * c->num_sms && rbf_bwd_smem_bytes(w.M, w.D_in) <= kRbfBwdSmemMax;
   const long nb = small ? Pp / kRbfCols : Pp / 128;
   const size_t smem = small ? rbf_bwd_smem_bytes(w.M, w.D_in) : ((size_t)w.M * w.D_in + kMaxD + 32) * sizeof(double);
   RC(dispatch_dmax(w.D_in, [&](auto dm) -> int {
     constexpr int DM = decltype(dm)::value;
     if (small) {
-      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
       LAUNCH((rbf_bwd2d_kernel<DM, false>), (unsigned)nb, 256, smem, r);
     } else {
-      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
       LAUNCH((rbf_bwd_kernel<DM, false>), (unsigned)nb, 128, smem, r);
     }
     return DGP_OK;
@@ -962,6 +968,8 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
   // the V-form adjoint pays ~8 extra M^3-class products per layer and step: worth it only when there are enough point-samples
   LateGuard late_guard{c};
   RC(prep_layers(c, model, lw, adj ? PREP_GRAD : (o.want_elbo ? PREP_KL : PREP_FWD), N * S >= c->vform_grad_min_ps, true));
+  for (const LayerWs& w : lw)   // refused in the planning pass, before any launch (the chunk loop below does not run there)
+    if (!moments_fit(c, w)) return DGP_ERR_UNSUPPORTED;
   const size_t base_used = c->used;
 
   int maxMp = 0, maxD = 1;

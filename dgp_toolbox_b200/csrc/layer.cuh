@@ -342,6 +342,10 @@ constexpr int kRbfCols = 64, kRbfRowGroups = 4;   // 256 threads: 64 point-sampl
 inline size_t rbf_bwd_smem_bytes(int M, int D_in) {
   return ((size_t)M * D_in + kMaxD + 32 + (size_t)kRbfRowGroups * kRbfCols * D_in) * sizeof(double);
 }
+// dynamic shared memory both kernel-adjoint variants opt into. The one-thread-per-column kernel needs at most
+// (768 * 31 + 64) * 8 B = 186.5 KiB; the row-group kernel's extra partial sums do not fit with large M * D_in (M = 640,
+// D_in = 31 needs 217.5 KiB), and such layers take the one-thread-per-column kernel at any size.
+constexpr size_t kRbfBwdSmemMax = 200 * 1024;
 
 // Small launches (fewer blocks than two waves of the one-thread-per-column kernel below): latency-bound, so each thread walks
 // every 4th inducing row of its column and the row groups' partial input gradients are summed through shared memory.

@@ -587,7 +587,9 @@ def natgrad_step(model: OModel, X, Y, zs, gamma: float, layer_indices: Sequence[
         g2 = 0.5 * (e2.grad + e2.grad.transpose(1, 2))
         theta1 = Sinv @ mu - gamma * e1.grad
         theta2 = -0.5 * Sinv - gamma * g2
-        S_new = torch.linalg.inv(-2.0 * theta2)
+        # one matrix at a time: with the MKL build of torch 2.11, a batched float64 torch.linalg.inv of 256 x 256 or larger after
+        # any torch.set_num_threads call stops in MKL ("Parameter 6 was incorrect on entry to DLASWP") and never returns
+        S_new = torch.stack([torch.linalg.inv(m) for m in -2.0 * theta2])
         S_new = 0.5 * (S_new + S_new.transpose(1, 2))
         out.append(((S_new @ theta1).squeeze(-1).T.contiguous(), torch.linalg.cholesky(S_new)))
     return out
