@@ -38,8 +38,6 @@ struct dgp_ctx {
   bool replay = false;                  // allocate as usual but launch nothing: the caller restores the region from a saved copy (dgp_svgp_from_k_cached)
   size_t ws_limit = (size_t)24 << 30;   // chunks of the minibatch are sized to stay under this
   int num_sms = 148;
-  int splitk_max = 64;                  // most splits of a contraction over the point-samples (sizes the split-K scratch)
-  int lower_waves = 9;                  // CTA waves a lower-only NT contraction is cut into (pick_splitk)
   bool chol_configured = false;
   int* d_info = nullptr;                // Cholesky failure flag
   // CUDA-graph replay of the ELBO+gradient step (dgp_set_graph): the step's launch sequence depends only on shapes, pointers
@@ -63,10 +61,9 @@ struct dgp_ctx {
   double* d_stage = nullptr;            // device side of that staging (outside the arena, which may be re-grown)
   size_t d_stage_bytes = 0;
   bool sync_launches = false;           // DGP_B200_SYNC_LAUNCHES: cudaDeviceSynchronize + error check after every launch (debugging)
+  bool vform_forward_calls = true;      // forward-only calls fold q_sqrt_d^T Lu^-T once per step and skip the A pass
   bool use_vform_grad = true;           // ... and so does the ELBO+gradient path (V-form adjoint in backward_layer)
-  bool vform_forward_calls = true;
   long vform_grad_min_ps = 32768;       // fewer point-samples than this: keep the A-form adjoint (no Cholesky-adjoint glue)
-  bool use_vform = true;                // forward-only calls fold q_sqrt_d^T Lu^-T once per step and skip the A pass
   bool share_first_layer = true;        // evaluate the first layer once per point instead of once per point-sample
   bool use_fused = true;                // fused conditional kernel (fused.cuh); false -> unfused GEMM pipeline
   bool use_fused_bwd = true;            // fused data-path adjoint (fused_bwd.cuh) for V-form layers it supports
@@ -258,6 +255,25 @@ int ensure_ws(dgp_ctx* c, size_t need) {
   return DGP_OK;
 }
 
+// Planning half of planned(): runs `pass` dry (it lays the arena out and launches nothing), then grows the arena to fit.
+template <typename F>
+int plan(dgp_ctx* c, F&& pass) {
+  c->dry = true; c->used = 0;
+  const int rc = pass();
+  c->dry = false;
+  if (rc != DGP_OK) return rc;
+  RC(ensure_ws(c, c->used));
+  c->used = 0;
+  return DGP_OK;
+}
+
+// Runs `pass` once to size the arena and once for real.
+template <typename F>
+int planned(dgp_ctx* c, F&& pass) {
+  RC(plan(c, pass));
+  return pass();
+}
+
 int gemm(dgp_ctx* c, GemmArgs g, bool nt) {
   if (c->dry || c->replay) return DGP_OK;
   ProfScope ps(c);
@@ -287,10 +303,12 @@ GemmArgs gargs(const double* A, long lda, const double* B, long ldb, double* C, 
 // Split-K count for a contraction over the point-samples: the count (<= 64, >= 8 k-tiles per chunk, partial tiles within
 // the scratch budget) whose CTA total fills whole waves best; ties go to the smaller count (less reduction traffic).
 constexpr size_t kSplitkPartDoubles = (size_t)96 << 20;   // 768 MB of split-K partial tiles at most
+constexpr int kSplitkMax = 64;    // most splits of a contraction over the point-samples (sizes the split-K scratch)
+constexpr int kLowerWaves = 9;    // CTA waves a lower-only NT contraction is cut into
 int pick_splitk(dgp_ctx* c, const GemmArgs& g, bool nt) {
   const GemmPlan p = gemm_plan(g, nt, c->num_sms);
   const size_t out_doubles = (size_t)g.batch * g.M * g.N;
-  long smax = c->splitk_max;
+  long smax = kSplitkMax;
   if ((size_t)smax * out_doubles > kSplitkPartDoubles) smax = (long)(kSplitkPartDoubles / out_doubles);
   const long ktiles = g.K / 16;
   if (smax > ktiles / 8) smax = ktiles / 8;
@@ -308,7 +326,7 @@ int pick_splitk(dgp_ctx* c, const GemmArgs& g, bool nt) {
   if (nt && g.c_lower && p.BM == 64 && gemm_small_bk32(g, nt)) {
     // lower-only NT product: its diagonal tiles run the 36-of-64-unit path and finish in ~0.56 of the time of the others, so
     // the CTAs are not uniform and many short CTAs pack better than whole waves of long ones (measured: 11 -> 33 splits, -10%)
-    long s = (c->lower_waves * (long)p.slots + p.tiles - 1) / p.tiles;
+    long s = (kLowerWaves * (long)p.slots + p.tiles - 1) / p.tiles;
     if (s > smax) s = smax;
     return (int)(s < 1 ? 1 : s);
   }
@@ -444,7 +462,34 @@ std::vector<PanelDesc> build_schedule(int Mp, int BM, int D_out, bool vform) {
 
 enum PrepLevel { PREP_FWD = 0, PREP_KL = 1, PREP_GRAD = 2 };
 
-int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& lw, PrepLevel level, bool vform_grad_ok = true,
+// What prep_layers lays out: the fused conditional kernel where a configuration fits (else the unfused GEMM pipeline), and the
+// V-form for the fused non-white layers (white layers are always V-form).
+struct LayerPath { bool fused, vform; };
+
+// The path the ctx's settings select for a model-level call at `level` over `point_samples` point-samples.
+LayerPath ctx_path(const dgp_ctx* c, PrepLevel level, long point_samples) {
+  // the V-form adjoint pays ~8 extra M^3-class products per layer and step: worth it only when there are enough point-samples
+  const bool vform = level == PREP_FWD ? c->vform_forward_calls
+                                       : level == PREP_GRAD && c->use_vform_grad && point_samples >= c->vform_grad_min_ps;
+  return {c->use_fused, vform};
+}
+
+// chol_inv_kernel / tri_inv_kernel opt in to the shared memory of the largest block they factorise (768), once per ctx (= device)
+int chol_smem_optin(dgp_ctx* c) {
+  if (c->chol_configured) return DGP_OK;
+  CK(cudaFuncSetAttribute(chol_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_smem_bytes(768)));
+  CK(cudaFuncSetAttribute(tri_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tri_inv_smem_bytes(768)));
+  c->chol_configured = true;
+  return DGP_OK;
+}
+
+// An M^3-class product whose K runs over the D_out blocks of Mp: few output tiles, long K, so split K over the blocks.
+void split_long_k(GemmArgs& g, int D, double* part) {
+  g.splitk = D >= 16 ? 16 : (D >= 2 ? D : 1);
+  g.part = part;
+}
+
+int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& lw, PrepLevel level, LayerPath path,
                 bool defer_late = false, const double* const* Ku_ext = nullptr) {
   const int nl = model->num_layers;
   lw.assign(nl, LayerWs());
@@ -470,7 +515,7 @@ int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& l
     }
     if (w.Mp > maxMp) maxMp = w.Mp;
     hargs[l] = CholArgs{w.Ku, w.L, nullptr, nullptr, w.Mp, c->d_info};   // inverse: tri_inv_kernel
-    w.fcfg = c->use_fused ? pick_fused_cfg(w.Mp, w.D_in, w.D_out) : -1;
+    w.fcfg = path.fused ? pick_fused_cfg(w.Mp, w.D_in, w.D_out) : -1;
     if (w.white && w.fcfg < 0) {
       c->err = "white=True layers run on the fused conditional kernel only (dgp_set_fused(1), and a layer shape it supports)";
       return DGP_ERR_UNSUPPORTED;
@@ -478,7 +523,7 @@ int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& l
     if (w.fcfg >= 0) {
       const int BM = kFusedChoices[w.fcfg].BM;
       const int nb = w.Mp / BM, kpb = BM / kPanelK;
-      w.vform = w.white || (level == PREP_FWD && c->use_vform && c->vform_forward_calls) || (level == PREP_GRAD && c->use_vform_grad && vform_grad_ok);
+      w.vform = w.white || path.vform;
       w.NP = ((w.vform ? 1 : 2) + w.D_out) * kpb * nb * (nb + 1) / 2;
       if (w.vform) { w.Cmat = walloc(c, mm * w.D_out); w.betaP = walloc(c, (size_t)w.Mp * 32); }
       if (w.vform && level == PREP_GRAD) {
@@ -521,15 +566,9 @@ int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& l
     LAUNCH(pad_params_kernel, (unsigned)((np + 255) / 256), 256, 0, d.q_sqrt, d.q_mu, w.M, w.Mp, w.D_out, w.RpT, w.Rcat, w.qmuP);
   }
   forkA.join();
-  {
-    if (!c->chol_configured) {   // per device (= per ctx)
-      CK(cudaFuncSetAttribute(chol_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_smem_bytes(768)));
-      c->chol_configured = true;
-    }
-    LAUNCH(chol_inv_kernel, nl, kCholThreads, chol_smem_bytes(maxMp), dargs);
-    CK(cudaFuncSetAttribute(tri_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tri_inv_smem_bytes(768)));
-    LAUNCH(tri_inv_kernel, dim3((unsigned)(maxMp / 32), (unsigned)nl), 256, tri_inv_smem_bytes(maxMp), dargs, dinv, dinvT);
-  }
+  RC(chol_smem_optin(c));
+  LAUNCH(chol_inv_kernel, nl, kCholThreads, chol_smem_bytes(maxMp), dargs);
+  LAUNCH(tri_inv_kernel, dim3((unsigned)(maxMp / 32), (unsigned)nl), 256, tri_inv_smem_bytes(maxMp), dargs, dinv, dinvT);
   LayerFork forkB(c, nl);
   for (int l = 0; l < nl; ++l) {   // operator stream of the fused conditional kernel
     forkB.use(l);
@@ -590,7 +629,7 @@ int prep_layers(dgp_ctx* c, const dgp_model_desc* model, std::vector<LayerWs>& l
         g = gargs(w.Kinv, Mp, w.Rcat, (long)D * Mp, w.KRcat, (long)D * Mp, Mp, D * Mp, Mp);  // Kinv [R_1 .. R_D]
         RC(gemm(c, g, false));
         g = gargs(w.KRcat, (long)D * Mp, w.KRcat, (long)D * Mp, w.KSK, Mp, Mp, Mp, D * Mp);   // sum_d (Kinv R_d)(Kinv R_d)^T
-        g.splitk = D >= 16 ? 16 : (D >= 2 ? D : 1); g.part = w.part_small;   // few output tiles, long K: split it
+        split_long_k(g, D, w.part_small);
         RC(gemm(c, g, true));
       }
     }
@@ -623,6 +662,22 @@ bool moments_fit(dgp_ctx* c, const LayerWs& w) {
   if (w.fcfg >= 0 || (size_t)w.M * w.D_out * sizeof(double) <= 160 * 1024) return true;
   c->err = "unfused conditional: M * D_out * 8 bytes of q_mu exceed the 160 KiB staged per CTA (fused path: M <= 256, D_out <= 16)";
   return false;
+}
+
+// ---- A-form GEMM pipeline of the conditional and its data-path adjoint, on [Mp][Pp] planes ----
+
+// V = Lu^-1 Kuf, A = Lu^-T V, T_d = q_sqrt_d^T A
+int aform_forward(dgp_ctx* c, const LayerWs& w, const double* K, double* V, double* A, double* T, long Pp) {
+  const int Mp = w.Mp;
+  GemmArgs g = gargs(w.Linv, Mp, K, Pp, V, Pp, Mp, (int)Pp, Mp);    // V = Lu^-1 Kuf            (layers.py:245)
+  g.a_tri = 1;
+  RC(gemm(c, g, false));
+  g = gargs(w.LinvT, Mp, V, Pp, A, Pp, Mp, (int)Pp, Mp);            // A = Lu^-T V              (layers.py:247)
+  g.a_tri = 2;
+  RC(gemm(c, g, false));
+  g = gargs(w.RpT, Mp, A, Pp, T, Pp, Mp, (int)Pp, Mp);              // T_d = q_sqrt_d^T A       (layers.py:257-271)
+  g.a_tri = 2; g.batch = w.D_out; g.sA = (long)Mp * Mp; g.sB = 0; g.sC = (long)Mp * Pp;
+  return gemm(c, g, false);
 }
 
 int forward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, ChunkLayer& cl, const Temps& tmp, bool stash,
@@ -675,15 +730,7 @@ int forward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, ChunkLa
   LAUNCH(kuf_kernel, dim3((unsigned)(Pp / kKufCols), (unsigned)(Mp / kKufRows)), 256, 0, cl.Xin, cl.xmod, d.Z, d.lengthscales,
          d.variance, w.M, Mp, w.D_in, P, Pp, K, d.kernel_kind);
   CAT(DGP_CAT_GEMM_FWD);
-  GemmArgs g = gargs(w.Linv, Mp, K, Pp, V, Pp, Mp, (int)Pp, Mp);    // V = Lu^-1 Kuf            (layers.py:245)
-  g.a_tri = 1;
-  RC(gemm(c, g, false));
-  g = gargs(w.LinvT, Mp, V, Pp, A, Pp, Mp, (int)Pp, Mp);            // A = Lu^-T V              (layers.py:247)
-  g.a_tri = 2;
-  RC(gemm(c, g, false));
-  g = gargs(w.RpT, Mp, A, Pp, T, Pp, Mp, (int)Pp, Mp);              // T_d = q_sqrt_d^T A       (layers.py:257-271)
-  g.a_tri = 2; g.batch = D; g.sA = (long)Mp * Mp; g.sB = 0; g.sC = (long)Mp * Pp;
-  RC(gemm(c, g, false));
+  RC(aform_forward(c, w, K, V, A, T, Pp));
 
   CAT(DGP_CAT_MOMENTS);
   MomentsArgs a;
@@ -750,6 +797,77 @@ int param_gemms(dgp_ctx* c, GemmArgs* gs, const bool* nts, int n, const ParamScr
   return DGP_OK;
 }
 
+// dA' = q_mu Gm^T + sum_d R_d (2 Gv_d o T_d), W = Ku^-1 dA'                          (SURVEY §9)
+// With `split` (split-K scratch shared with the parameter contractions still in flight), few point-samples deal the D blocks of
+// the second product out to splits.
+int aform_adjoint(dgp_ctx* c, const LayerWs& w, const double* T, const double* GmPad, const double* GvT, double* dA, double* W,
+                  long Pp, const ParamScratch* split) {
+  const int Mp = w.Mp, D = w.D_out;
+  GemmArgs g = gargs(w.qmuP, 32, GmPad, 32, dA, Pp, Mp, (int)Pp, 32);
+  RC(gemm(c, g, true));
+  g = gargs(w.Rcat, (long)D * Mp, T, Pp, dA, Pp, Mp, (int)Pp, D * Mp);
+  g.a_tri = 1; g.kblocks = D; g.kblk = Mp; g.bscale = GvT; g.ld_bscale = Pp; g.bscale_mul = 2.0; g.beta = 1.0;
+  if (D == 1) g.kblocks = 1;
+  if (split && D > 1) {
+    // few point-samples (a shared first layer): too few output tiles to occupy the GPU, so deal the D blocks out to splits
+    const GemmPlan p = gemm_plan(g, false, c->num_sms);
+    long s = p.tiles > 0 ? p.slots / (2 * p.tiles) : 1;
+    if (s > D) s = D;
+    if (s >= 2 && (size_t)s * Mp * Pp <= split->cap) {
+      join_param(c, 0); join_param(c, 1);   // the scratch is shared with the parameter contractions still in flight
+      g.splitk = (int)s; g.part = split->part;
+    }
+  }
+  RC(gemm(c, g, false));
+  g = gargs(w.Kinv, Mp, dA, Pp, W, Pp, Mp, (int)Pp, Mp);
+  return gemm(c, g, false);
+}
+
+// The contractions over the point-samples that give the data parts of dKu, dq_sqrt and dq_mu (NT flags in kAformParamNT),
+// accumulated onto the previous chunks' with `beta`.
+constexpr bool kAformParamNT[3] = {true, true, false};
+void aform_param_args(const LayerWs& w, const double* W, const double* A, const double* T, const double* GvT, const double* GmPad,
+                      long Pp, double beta, GemmArgs pg[3]) {
+  const int Mp = w.Mp;
+  pg[0] = gargs(W, Pp, A, Pp, w.dKu, Mp, Mp, Mp, (int)Pp);          // dKu (data part) = -Wg A^T
+  pg[0].alpha = -1.0; pg[0].beta = beta;
+  pg[1] = gargs(A, Pp, T, Pp, w.dR, Mp, Mp, Mp, (int)Pp);           // dq_sqrt_d (data part) = tril(A diag(2 Gv_d) T_d^T)
+  pg[1].alpha = 2.0; pg[1].beta = beta; pg[1].batch = w.D_out; pg[1].sA = 0; pg[1].sB = (long)Mp * Pp; pg[1].sC = (long)Mp * Mp;
+  pg[1].c_lower = 1; pg[1].kscale = GvT; pg[1].sScale = Pp;
+  pg[2] = gargs(A, Pp, GmPad, 32, w.dqmu, 32, Mp, 32, (int)Pp);     // dq_mu (data part) = A Gm
+  pg[2].beta = beta;
+}
+
+// RBF adjoint on the Kuf block: W -> Wg (in place), Gbar, dXin, [X,1], partial sums for dl / ds2. VF: W is K-bar = dELBO/dKuf of
+// the V-form and A is null; otherwise W = Ku^-1 dA' and A the stashed A plane. Sets `nb` to the blocks launched (one row of
+// partial sums each, for reduce_partials_kernel).
+template <bool VF>
+int kernel_adjoint(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const ChunkLayer& cl, const Upstream& up, double* W,
+                   const double* A, double* Gbar, double* dXin, double* XaugPad, double* rbf_part, long P, long& nb) {
+  const long Pp = round_up(P, kTileP);
+  CAT(DGP_CAT_RBF_BWD);
+  RbfBwdArgs r;
+  memset(&r, 0, sizeof(r));
+  r.W = W; r.A = A; r.gq = up.gq; r.Gbar = Gbar; r.Xin = cl.Xin; r.xmod = cl.xmod; r.Z = d.Z; r.ls = d.lengthscales;
+  r.var = d.variance; r.M = w.M; r.Mp = w.Mp; r.D_in = w.D_in; r.P = P; r.Pp = Pp; r.Gm = up.Gm; r.D_out = w.D_out;
+  r.mean_kind = d.mean_kind; r.mfW = d.mf_W; r.kind = d.kernel_kind; r.dXin = dXin; r.XaugPad = XaugPad; r.part = rbf_part;
+  // latency-bound launch: 64-column blocks with 4 row groups, where their shared memory fits
+  const bool small = Pp / 128 < 2L * c->num_sms && rbf_bwd_smem_bytes(w.M, w.D_in) <= kRbfBwdSmemMax;
+  nb = small ? Pp / kRbfCols : Pp / 128;
+  const size_t smem = small ? rbf_bwd_smem_bytes(w.M, w.D_in) : ((size_t)w.M * w.D_in + kMaxD + 32) * sizeof(double);
+  return dispatch_dmax(w.D_in, [&](auto dm) -> int {
+    constexpr int DM = decltype(dm)::value;
+    if (small) {
+      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, VF>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
+      LAUNCH((rbf_bwd2d_kernel<DM, VF>), (unsigned)nb, 256, smem, r);
+    } else {
+      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, VF>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
+      LAUNCH((rbf_bwd_kernel<DM, VF>), (unsigned)nb, 128, smem, r);
+    }
+    return DGP_OK;
+  });
+}
+
 int backward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const ChunkLayer& cl, const Temps& tmp,
                    const Upstream& up, double* dXin, double* XaugPad, double* rbf_part, const ParamScratch& ps, long Nc, long S, bool first_chunk,
                    bool params = true) {
@@ -803,27 +921,7 @@ int backward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const 
     g = gargs(w.LinvT, Mp, dV, Pp, Kbar, Pp, Mp, (int)Pp, Mp);
     g.a_tri = 2;
     RC(gemm(c, g, false));
-    CAT(DGP_CAT_RBF_BWD);
-    RbfBwdArgs r;
-    memset(&r, 0, sizeof(r));
-    r.W = Kbar; r.A = nullptr; r.gq = up.gq; r.Gbar = Gbar; r.Xin = cl.Xin; r.xmod = cl.xmod; r.Z = d.Z; r.ls = d.lengthscales;
-    r.var = d.variance; r.M = w.M; r.Mp = Mp; r.D_in = w.D_in; r.P = P; r.Pp = Pp; r.Gm = up.Gm; r.D_out = D;
-    r.mean_kind = d.mean_kind; r.mfW = d.mf_W; r.kind = d.kernel_kind; r.dXin = dXin; r.XaugPad = XaugPad; r.part = rbf_part;
-    // latency-bound launch: 64-column blocks with 4 row groups, where their shared memory fits
-    const bool small = Pp / 128 < 2L * c->num_sms && rbf_bwd_smem_bytes(w.M, w.D_in) <= kRbfBwdSmemMax;
-    nbv = small ? Pp / kRbfCols : Pp / 128;
-    const size_t smemv = small ? rbf_bwd_smem_bytes(w.M, w.D_in) : ((size_t)w.M * w.D_in + kMaxD + 32) * sizeof(double);
-    RC(dispatch_dmax(w.D_in, [&](auto dm) -> int {
-      constexpr int DM = decltype(dm)::value;
-      if (small) {
-        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
-        LAUNCH((rbf_bwd2d_kernel<DM, true>), (unsigned)nbv, 256, smemv, r);
-      } else {
-        if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
-        LAUNCH((rbf_bwd_kernel<DM, true>), (unsigned)nbv, 128, smemv, r);
-      }
-      return DGP_OK;
-    }));
+    RC(kernel_adjoint<true>(c, d, w, cl, up, Kbar, nullptr, Gbar, dXin, XaugPad, rbf_part, P, nbv));
     }
     if (!params) return DGP_OK;
     CAT(DGP_CAT_GEMM_BWD_PARAM);
@@ -850,64 +948,16 @@ int backward_layer(dgp_ctx* c, const dgp_layer_desc& d, const LayerWs& w, const 
     }));
     return DGP_OK;
   }
-  // dA' = q_mu Gm^T + sum_d R_d (2 Gv_d o T_d)                                       (SURVEY §9)
   CAT(DGP_CAT_GEMM_BWD_DATA);
-  GemmArgs g = gargs(w.qmuP, 32, up.GmPad, 32, dA, Pp, Mp, (int)Pp, 32);
-  RC(gemm(c, g, true));
-  g = gargs(w.Rcat, (long)D * Mp, cl.T, Pp, dA, Pp, Mp, (int)Pp, D * Mp);
-  g.a_tri = 1; g.kblocks = D; g.kblk = Mp; g.bscale = up.GvT; g.ld_bscale = Pp; g.bscale_mul = 2.0; g.beta = 1.0;
-  if (D == 1) { g.kblocks = 1; }
-  if (D > 1) {
-    // few point-samples (a shared first layer): too few output tiles to occupy the GPU, so deal the D blocks out to splits
-    const GemmPlan p = gemm_plan(g, false, c->num_sms);
-    long s = p.tiles > 0 ? p.slots / (2 * p.tiles) : 1;
-    if (s > D) s = D;
-    if (s >= 2 && (size_t)s * Mp * Pp <= ps.cap) {
-      join_param(c, 0); join_param(c, 1);   // the scratch is shared with the parameter contractions still in flight
-      g.splitk = (int)s; g.part = ps.part;
-    }
-  }
-  RC(gemm(c, g, false));
-  // W = Ku^-1 dA'
-  g = gargs(w.Kinv, Mp, dA, Pp, W, Pp, Mp, (int)Pp, Mp);
-  RC(gemm(c, g, false));
-  // RBF adjoint on the Kuf block: W -> Wg (in place), Gbar, dXin, [X,1], partial sums for dl / ds2
-  CAT(DGP_CAT_RBF_BWD);
-  RbfBwdArgs r;
-  memset(&r, 0, sizeof(r));
-  r.W = W; r.A = cl.A; r.gq = up.gq; r.Gbar = Gbar; r.Xin = cl.Xin; r.xmod = cl.xmod; r.Z = d.Z; r.ls = d.lengthscales;
-  r.var = d.variance; r.M = w.M; r.Mp = Mp; r.D_in = w.D_in; r.P = P; r.Pp = Pp; r.Gm = up.Gm; r.D_out = D;
-  r.mean_kind = d.mean_kind; r.mfW = d.mf_W; r.kind = d.kernel_kind; r.dXin = dXin; r.XaugPad = XaugPad; r.part = rbf_part;
-  // latency-bound launch: 64-column blocks with 4 row groups, where their shared memory fits
-  const bool small = Pp / 128 < 2L * c->num_sms && rbf_bwd_smem_bytes(w.M, w.D_in) <= kRbfBwdSmemMax;
-  const long nb = small ? Pp / kRbfCols : Pp / 128;
-  const size_t smem = small ? rbf_bwd_smem_bytes(w.M, w.D_in) : ((size_t)w.M * w.D_in + kMaxD + 32) * sizeof(double);
-  RC(dispatch_dmax(w.D_in, [&](auto dm) -> int {
-    constexpr int DM = decltype(dm)::value;
-    if (small) {
-      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd2d_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
-      LAUNCH((rbf_bwd2d_kernel<DM, false>), (unsigned)nb, 256, smem, r);
-    } else {
-      if (!c->dry) CK(cudaFuncSetAttribute((rbf_bwd_kernel<DM, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRbfBwdSmemMax));
-      LAUNCH((rbf_bwd_kernel<DM, false>), (unsigned)nb, 128, smem, r);
-    }
-    return DGP_OK;
-  }));
+  RC(aform_adjoint(c, w, cl.T, up.GmPad, up.GvT, dA, W, Pp, &ps));
+  long nb = 0;
+  RC(kernel_adjoint<false>(c, d, w, cl, up, W, cl.A, Gbar, dXin, XaugPad, rbf_part, P, nb));
   if (!params) return DGP_OK;   // input gradient only (acquisition): the contractions over the point-samples are not needed
   CAT(DGP_CAT_GEMM_BWD_PARAM);
   GemmArgs pg[4];
-  const bool pnt[4] = {true, true, false, false};
-  // dKu (data part) = -Wg A^T
-  pg[0] = gargs(W, Pp, cl.A, Pp, w.dKu, Mp, Mp, Mp, (int)Pp);
-  pg[0].alpha = -1.0; pg[0].beta = beta;
-  // dq_sqrt_d (data part) = tril(A diag(2 Gv_d) T_d^T)
-  pg[1] = gargs(cl.A, Pp, cl.T, Pp, w.dR, Mp, Mp, Mp, (int)Pp);
-  pg[1].alpha = 2.0; pg[1].beta = beta; pg[1].batch = D; pg[1].sA = 0; pg[1].sB = (long)Mp * Pp; pg[1].sC = (long)Mp * Mp; pg[1].c_lower = 1;
-  pg[1].kscale = up.GvT; pg[1].sScale = Pp;
-  // dq_mu (data part) = A Gm ;  H = Gbar [X, 1]
-  pg[2] = gargs(cl.A, Pp, up.GmPad, 32, w.dqmu, 32, Mp, 32, (int)Pp);
-  pg[2].beta = beta;
-  pg[3] = gargs(Gbar, Pp, XaugPad, 32, w.H, 32, Mp, 32, (int)Pp);
+  const bool pnt[4] = {kAformParamNT[0], kAformParamNT[1], kAformParamNT[2], false};
+  aform_param_args(w, W, cl.A, cl.T, up.GvT, up.GmPad, Pp, beta, pg);
+  pg[3] = gargs(Gbar, Pp, XaugPad, 32, w.H, 32, Mp, 32, (int)Pp);   // H = Gbar [X, 1]
   pg[3].beta = beta;
   RC(param_gemms(c, pg, pnt, 4, ps, nullptr, [&]() -> int {
     LAUNCH(reduce_partials_kernel, w.D_in + 1, 256, 0, rbf_part, nb, w.D_in + 1, w.rbf_red, first_chunk ? 0 : 1);
@@ -934,29 +984,35 @@ struct RunOpts {
 
 // Split-K scratch of the adjoint: four regions (the parameter contractions of a layer run side by side), sized for the widest
 // layer so that the same layout serves every layer.
-void splitk_regions(const dgp_ctx* c, const std::vector<LayerWs>& lw, size_t room[4]) {
+void splitk_regions(const std::vector<LayerWs>& lw, size_t room[4]) {
   size_t Mp = 0, D = 1;
   for (const LayerWs& w : lw) {
     if ((size_t)w.Mp > Mp) Mp = w.Mp;
     if ((size_t)w.D_out > D) D = w.D_out;
   }
-  const size_t sm = (size_t)c->splitk_max;
+  const size_t sm = kSplitkMax;
   room[0] = sm * Mp * Mp; room[1] = sm * D * Mp * Mp; room[2] = sm * Mp * 32; room[3] = sm * Mp * 32;
 }
-size_t max_splitk_part(const dgp_ctx* c, const std::vector<LayerWs>& lw) {
+size_t max_splitk_part(const std::vector<LayerWs>& lw) {
   size_t room[4];
-  splitk_regions(c, lw, room);
+  splitk_regions(lw, room);
   const size_t m = room[0] + room[1] + room[2] + room[3] + 1024;
   return m < kSplitkPartDoubles ? m : kSplitkPartDoubles + ((size_t)32 * 1024 * 1024 / 8);
+}
+
+int check_chain(dgp_ctx* c, const dgp_model_desc* model, long N, long S) {
+  const int nl = model->num_layers;
+  if (nl < 1 || N < 1 || S < 1) { c->err = "need num_layers >= 1, N >= 1, S >= 1"; return DGP_ERR_ARG; }
+  for (int l = 1; l < nl; ++l)
+    if (model->layers[l].D_in != model->layers[l - 1].D_out) { c->err = "layer widths do not chain"; return DGP_ERR_ARG; }
+  return DGP_OK;
 }
 
 // Runs the chain over all chunks. Returns via opts outputs. `plan` semantics are handled by c->dry.
 int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, long S, unsigned long long seed, long n_offset,
               RunOpts& o) {
+  RC(check_chain(c, model, N, S));
   const int nl = model->num_layers;
-  if (nl < 1 || N < 1 || S < 1) { c->err = "need num_layers >= 1, N >= 1, S >= 1"; return DGP_ERR_ARG; }
-  for (int l = 1; l < nl; ++l)
-    if (model->layers[l].D_in != model->layers[l - 1].D_out) { c->err = "layer widths do not chain"; return DGP_ERR_ARG; }
   const bool grad = o.want_grad;
   const bool adj = grad || o.dx;   // the adjoint chain runs (needs the A / T_d stash and Ku^-1)
   // first-layer sharing (see expand_first_layer_kernel): needs a later layer to consume the per-sample draws
@@ -965,9 +1021,9 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
   if ((grad || o.want_elbo) && !model->lik_variance) { c->err = "lik_variance is null"; return DGP_ERR_ARG; }
 
   std::vector<LayerWs> lw;
-  // the V-form adjoint pays ~8 extra M^3-class products per layer and step: worth it only when there are enough point-samples
   LateGuard late_guard{c};
-  RC(prep_layers(c, model, lw, adj ? PREP_GRAD : (o.want_elbo ? PREP_KL : PREP_FWD), N * S >= c->vform_grad_min_ps, true));
+  const PrepLevel level = adj ? PREP_GRAD : (o.want_elbo ? PREP_KL : PREP_FWD);
+  RC(prep_layers(c, model, lw, level, ctx_path(c, level, N * S), true));
   for (const LayerWs& w : lw)   // refused in the planning pass, before any launch (the chunk loop below does not run there)
     if (!moments_fit(c, w)) return DGP_ERR_UNSUPPORTED;
   const size_t base_used = c->used;
@@ -985,7 +1041,7 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
   if (!adj) pp_doubles += (size_t)maxD * maxMp;                      // shared T
   if (adj) pp_doubles += 2 * (size_t)maxD + 32 + 1 + 32 + 2 * 32;    // Gm, GvT, GmPad, gq, XaugPad, dX ping-pong
   if (adj && nl > 1) pp_doubles += 3 * (size_t)maxMp + 2 * (size_t)maxD + 32 + 1 + 32;   // second set of adjoint temporaries
-  size_t fixed = base_used + (adj ? max_splitk_part(c, lw) * sizeof(double) : 0) + ((size_t)8 << 20);
+  size_t fixed = base_used + (adj ? max_splitk_part(lw) * sizeof(double) : 0) + ((size_t)8 << 20);
   long Nc_max;
   {
     size_t avail = c->ws_limit > fixed ? c->ws_limit - fixed : 0;
@@ -1038,7 +1094,7 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
     dXa = walloc(c, (size_t)Ppmax * 32);
     dXb = walloc(c, (size_t)Ppmax * 32);
     rbf_part = walloc(c, (size_t)nbmax * 8 * 20);   // one row of partials per 64-column block of rbf_bwd_kernel
-    skcap = max_splitk_part(c, lw);
+    skcap = max_splitk_part(lw);
     skpart = walloc(c, skcap);
     if (nl > 1) {   // second set: layer l's parameter contractions read theirs while layer l-1's data path fills the other
       tmp1.t0 = walloc(c, (size_t)maxMp * Ppmax);
@@ -1055,7 +1111,7 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
   ParamScratch ps;
   ps.part = skpart; ps.cap = skcap;
   if (adj) {
-    splitk_regions(c, lw, ps.room);
+    splitk_regions(lw, ps.room);
     ps.off[0] = 0; ps.off[1] = ps.room[0]; ps.off[2] = ps.off[1] + ps.room[1]; ps.off[3] = ps.off[2] + ps.room[2];
     ps.fixed = ps.off[3] + ps.room[3] <= skcap;
   }
@@ -1231,7 +1287,7 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
           g.batch = D; g.sA = Mp; g.sB = Mp; g.sC = Mp;
           RC(gemm(c, g, false));
           g = gargs(w.CTcat, (long)D * Mp, w.DCt, (long)D * Mp, w.G1, Mp, Mp, Mp, D * Mp);
-          g.splitk = D >= 16 ? 16 : (D >= 2 ? D : 1); g.part = w.part_small;   // few output tiles, long K: split it
+          split_long_k(g, D, w.part_small);
           RC(gemm(c, g, true));
           g = gargs(w.betaP, 32, w.dbeta, 32, w.G1, Mp, Mp, Mp, 32);
           g.beta = 1.0;
@@ -1252,7 +1308,7 @@ int run_model(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, 
           if (!w.white) {
             g = gargs(w.DCt, (long)D * Mp, w.RpT, Mp, w.dLinv, Mp, Mp, Mp, D * Mp);
             g.beta = 1.0;
-            g.splitk = D >= 16 ? 16 : (D >= 2 ? D : 1); g.part = w.part_small;
+            split_long_k(g, D, w.part_small);
             RC(gemm(c, g, false));
             g = gargs(w.dbeta, 32, w.qmuP, 32, w.dLinv, Mp, Mp, Mp, 32);
             g.beta = 1.0;
@@ -1324,7 +1380,7 @@ std::vector<unsigned char> graph_key(dgp_ctx* c, const dgp_model_desc* model, co
   key_put(k, o.want_grad); key_put(k, o.want_elbo); key_put(k, o.Y); key_put(k, o.Dy); key_put(k, o.scale); key_put(k, o.kl_weight);
   key_put(k, o.out_flat); key_put(k, o.ve); key_put(k, o.pm); key_put(k, o.pv); key_put(k, o.add_lik); key_put(k, o.ei); key_put(k, o.y_min);
   key_put(k, o.ei_analytic); key_put(k, o.need_last_sample); key_put(k, o.dx); key_put(k, o.acq_kind); key_put(k, o.acq_add_lik);
-  key_put(k, c->use_fused); key_put(k, c->use_vform); key_put(k, c->use_vform_grad); key_put(k, c->vform_forward_calls);
+  key_put(k, c->use_fused); key_put(k, c->use_vform_grad); key_put(k, c->vform_forward_calls);
   key_put(k, c->vform_grad_min_ps); key_put(k, c->share_first_layer); key_put(k, c->parallel_layers); key_put(k, c->ws_limit);
   return k;
 }
@@ -1339,12 +1395,8 @@ int run_model_graphed(dgp_ctx* c, const dgp_model_desc* model, const double* X, 
   for (auto& g : c->graphs)
     if (g.key == key) { hit = &g; break; }
   if (!hit) {
-    c->dry = true; c->used = 0;
-    int rc = run_model(c, model, X, N, S, seed, n_offset, o);
-    c->dry = false;
-    if (rc != DGP_OK) return rc;
-    RC(ensure_ws(c, c->used));   // may drop every cached graph (their nodes point into the old arena)
-    c->used = 0;
+    // growing the arena may drop every cached graph (their nodes point into the old arena)
+    RC(plan(c, [&] { return run_model(c, model, X, N, S, seed, n_offset, o); }));
     if (!c->cap_stream) CK(cudaStreamCreateWithFlags(&c->cap_stream, cudaStreamNonBlocking));
     if (!c->d_seed) CK(cudaMalloc(&c->d_seed, sizeof(unsigned long long)));
     if (c->graphs.size() >= kMaxGraphs) {   // evict the least recently used entry
@@ -1362,7 +1414,7 @@ int run_model_graphed(dgp_ctx* c, const dgp_model_desc* model, const double* X, 
     const long launches0 = c->launches;
     CK(cudaStreamBeginCapture(c->cap_stream, cudaStreamCaptureModeRelaxed));
     c->stream = c->cap_stream; c->seed_ptr = c->d_seed; c->keep = &e.pinned;
-    rc = run_model(c, model, X, N, S, seed, n_offset, o);
+    int rc = run_model(c, model, X, N, S, seed, n_offset, o);
     c->stream = user; c->seed_ptr = nullptr; c->keep = nullptr;
     cudaGraph_t graph = nullptr;
     cudaError_t ce = cudaStreamEndCapture(c->cap_stream, &graph);
@@ -1396,14 +1448,7 @@ int run_model_planned(dgp_ctx* c, const dgp_model_desc* model, const double* X, 
   CK(cudaSetDevice(c->device));
   if (c->use_graph && !c->profiling && !o.io.zs && !o.io.Fs && !o.io.Fmeans && !o.io.Fvars)
     return run_model_graphed(c, model, X, N, S, seed, n_offset, o);
-  c->dry = true; c->used = 0;
-  int rc = run_model(c, model, X, N, S, seed, n_offset, o);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  RC(run_model(c, model, X, N, S, seed, n_offset, o));
-  return DGP_OK;
+  return planned(c, [&] { return run_model(c, model, X, N, S, seed, n_offset, o); });
 }
 
 int check_chol(dgp_ctx* c) {
@@ -1535,8 +1580,6 @@ int dgp_ctx_create(int device, void* cuda_stream, dgp_ctx** out) {
   if (const char* e = getenv("DGP_B200_SKEW")) c->group_skew = atoi(e);
   c->stream = reinterpret_cast<cudaStream_t>(cuda_stream);
   if (cudaMalloc(&c->d_info, sizeof(int)) != cudaSuccess || cudaMemset(c->d_info, 0, sizeof(int)) != cudaSuccess) { delete c; return DGP_ERR_CUDA; }
-  if (const char* e = getenv("DGP_B200_SPLITK_MAX")) { const int v = atoi(e); if (v >= 1 && v <= 512) c->splitk_max = v; }
-  if (const char* e = getenv("DGP_B200_LOWER_WAVES")) { const int v = atoi(e); if (v >= 1 && v <= 256) c->lower_waves = v; }
   const char* lim = getenv("DGP_B200_WS_GB");
   if (lim && atof(lim) > 0.0) c->ws_limit = (size_t)(atof(lim) * (double)((size_t)1 << 30));
   *out = c;
@@ -1589,7 +1632,6 @@ int dgp_set_parallel_layers(dgp_ctx* c, int on) {
 
 int dgp_set_vform(dgp_ctx* c, int forward_calls, int gradient_calls) {
   if (!c) return DGP_ERR_ARG;
-  c->use_vform = forward_calls != 0 || gradient_calls != 0;
   c->use_vform_grad = gradient_calls != 0;
   c->vform_grad_min_ps = gradient_calls == 2 ? 0 : 32768;   // 2: always, 1: only with enough point-samples to amortise the glue
   c->vform_forward_calls = forward_calls != 0;
@@ -1689,13 +1731,7 @@ int dgp_kuu_chol(dgp_ctx* c, const dgp_layer_desc* layer, double* Ku_out, double
   CK(cudaSetDevice(c->device));
   dgp_model_desc m{1, layer, nullptr};
   std::vector<LayerWs> lw;
-  c->dry = true; c->used = 0;
-  int rc = prep_layers(c, &m, lw, PREP_FWD);
-  c->dry = false;
-  RC(rc);
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  RC(prep_layers(c, &m, lw, PREP_FWD));
+  RC(planned(c, [&] { return prep_layers(c, &m, lw, PREP_FWD, ctx_path(c, PREP_FWD, 0)); }));
   const long mm = (long)layer->M * layer->M;
   if (Ku_out) LAUNCH(unpad_square_kernel, (unsigned)((mm + 255) / 256), 256, 0, lw[0].Ku, lw[0].M, lw[0].Mp, Ku_out);
   if (Lu_out) LAUNCH(unpad_square_kernel, (unsigned)((mm + 255) / 256), 256, 0, lw[0].L, lw[0].M, lw[0].Mp, Lu_out);
@@ -1707,13 +1743,7 @@ int dgp_kl(dgp_ctx* c, const dgp_layer_desc* layer, double* kl_out) {
   CK(cudaSetDevice(c->device));
   dgp_model_desc m{1, layer, nullptr};
   std::vector<LayerWs> lw;
-  c->dry = true; c->used = 0;
-  int rc = prep_layers(c, &m, lw, PREP_KL);
-  c->dry = false;
-  RC(rc);
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  RC(prep_layers(c, &m, lw, PREP_KL));
+  RC(planned(c, [&] { return prep_layers(c, &m, lw, PREP_KL, ctx_path(c, PREP_KL, 0)); }));
   CK(cudaMemcpyAsync(kl_out, lw[0].kl, sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
   return check_chol(c);
 }
@@ -1744,18 +1774,12 @@ namespace {
 int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, long S, const double* const* zs_host,
                  unsigned long long seed, long n_offset, double* const* Fs_host, double* const* Fmeans_host,
                  double* const* Fvars_host) {
+  RC(check_chain(c, model, N, S));
   const int nl = model->num_layers;
-  if (nl < 1 || N < 1 || S < 1) { c->err = "need num_layers >= 1, N >= 1, S >= 1"; return DGP_ERR_ARG; }
-  for (int l = 1; l < nl; ++l)
-    if (model->layers[l].D_in != model->layers[l - 1].D_out) { c->err = "layer widths do not chain"; return DGP_ERR_ARG; }
   const long Np = round_up(N, kTileM);
   if (Np > 768) { c->err = "full_cov=True: N > 768 is not supported (one CTA factorises an N x N block)"; return DGP_ERR_UNSUPPORTED; }
   std::vector<LayerWs> lw;
-  const bool vf_saved = c->use_vform, vfc_saved = c->vform_forward_calls;
-  c->use_vform = true; c->vform_forward_calls = true;      // the covariance blocks are built from the V-form planes
-  int rc = prep_layers(c, model, lw, PREP_FWD);
-  c->use_vform = vf_saved; c->vform_forward_calls = vfc_saved;
-  RC(rc);
+  RC(prep_layers(c, model, lw, PREP_FWD, {c->use_fused, true}));   // the covariance blocks are built from the V-form planes
   const long P = N * S, Pp = round_up(P, kTileP);
   int maxD = 1;
   for (int l = 0; l < nl; ++l) {
@@ -1782,10 +1806,7 @@ int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long 
   std::vector<CholArgs> hargs(nblk);
   for (size_t i = 0; i < nblk; ++i) hargs[i] = CholArgs{cin + i * Np * Np, Lf + i * Np * Np, nullptr, nullptr, (int)Np, c->d_info};
   H2D(dargs, hargs.data(), sizeof(CholArgs) * nblk);
-  if (!c->chol_configured) {
-    CK(cudaFuncSetAttribute(chol_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_smem_bytes(768)));
-    c->chol_configured = true;
-  }
+  RC(chol_smem_optin(c));
   for (int l = 0; l < nl; ++l) {
     const dgp_layer_desc& d = model->layers[l];
     const LayerWs& w = lw[l];
@@ -1826,13 +1847,7 @@ int dgp_propagate_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double
                            double* const* Fmeans_host, double* const* Fvars_host) {
   if (!c || !model || !X) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  c->dry = true; c->used = 0;
-  int rc = run_full_cov(c, model, X, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  RC(run_full_cov(c, model, X, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host));
+  RC(planned(c, [&] { return run_full_cov(c, model, X, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host); }));
   return check_chol(c);
 }
 
@@ -1854,30 +1869,34 @@ int comp_check(dgp_ctx* c, const dgp_comp_kernel* k) {
   return DGP_OK;
 }
 
-// The layer's conditional (and, with Gm, its adjoint) on supplied kernel matrices: A-form GEMM pipeline, one pass over all P.
-int svgp_from_k_run(dgp_ctx* c, int M, int D, long P, const double* Ku, const double* Kuf, const double* Kdiag, const double* q_mu,
-                    const double* q_sqrt, double* mean, double* var, double* kl, const double* Gm, const double* Gv, double gkl,
-                    double* dKu, double* dKuf, double* dKdiag, double* dq_mu, double* dq_sqrt, double* cache = nullptr,
-                    size_t cache_bytes = 0, bool cache_load = false, double* stash = nullptr) {
-  const bool grad = Gm != nullptr;
+// Prep of the supplied-matrix path: one layer on the A-form GEMM pipeline, Kuu = the caller's Ku. This also lays out the region
+// that dgp_svgp_prep_cache_bytes sizes and the cached calls copy.
+int svgp_prep(dgp_ctx* c, int M, int D, const double* Ku, const double* q_mu, const double* q_sqrt, PrepLevel level,
+              std::vector<LayerWs>& lw) {
   // a descriptor that satisfies check_layer: the kernel fields are never read (Ku is supplied, the fused kernels are off)
   dgp_layer_desc d;
   memset(&d, 0, sizeof(d));
   d.D_in = 1; d.D_out = D; d.M = M; d.white = 0; d.mean_kind = 0; d.kernel_kind = 0;
   d.Z = Ku; d.lengthscales = Ku; d.variance = Ku; d.q_mu = q_mu; d.q_sqrt = q_sqrt; d.jitter = 0.0;
   dgp_model_desc model{1, &d, nullptr};
-  std::vector<LayerWs> lw;
-  const bool fused_saved = c->use_fused;
-  c->use_fused = false;
   const double* kext[1] = {Ku};
+  return prep_layers(c, &model, lw, level, {false, false}, false, kext);
+}
+
+// The layer's conditional (and, with Gm, its adjoint) on supplied kernel matrices: A-form GEMM pipeline, one pass over all P.
+int svgp_from_k_run(dgp_ctx* c, int M, int D, long P, const double* Ku, const double* Kuf, const double* Kdiag, const double* q_mu,
+                    const double* q_sqrt, double* mean, double* var, double* kl, const double* Gm, const double* Gv, double gkl,
+                    double* dKu, double* dKuf, double* dKdiag, double* dq_mu, double* dq_sqrt, double* cache = nullptr,
+                    size_t cache_bytes = 0, bool cache_load = false, double* stash = nullptr) {
+  const bool grad = Gm != nullptr;
+  std::vector<LayerWs> lw;
   // With a cache the per-layer replicated work (Kuu factorisation, inverse, the M^3 products, KL) is done ONCE for all applications
   // of the layer inside one ELBO evaluation and their adjoints: the first call stores the prepared region of the arena, the others
   // lay the region out again without launching anything and copy it back (a few MB, device to device).
   const size_t prep_start = c->used;
   c->replay = cache != nullptr && cache_load;
-  int rc = prep_layers(c, &model, lw, (grad || cache) ? PREP_GRAD : PREP_KL, false, false, kext);
+  const int rc = svgp_prep(c, M, D, Ku, q_mu, q_sqrt, (grad || cache) ? PREP_GRAD : PREP_KL, lw);
   c->replay = false;
-  c->use_fused = fused_saved;
   RC(rc);
   if (cache && !c->dry) {
     const size_t prep_bytes = c->used - prep_start;
@@ -1905,24 +1924,15 @@ int svgp_from_k_run(dgp_ctx* c, int M, int D, long P, const double* Ku, const do
   if (grad) {
     dA = walloc(c, plane); W = walloc(c, plane);
     GvT = walloc(c, (size_t)D * Pp); GmPad = walloc(c, (size_t)Pp * 32); gq = walloc(c, (size_t)Pp);
-    partcap = max_splitk_part(c, lw);
+    partcap = max_splitk_part(lw);
     part = walloc(c, partcap);
     dummy = walloc(c, 64);
   }
   if (c->dry) return DGP_OK;
   CAT(DGP_CAT_GEMM_FWD);
-  GemmArgs g;
   if (!reuse) {
     LAUNCH(pad_plane_kernel, (unsigned)((plane + 255) / 256), 256, 0, Kuf, M, Mp, P, Pp, K);
-    g = gargs(w.Linv, Mp, K, Pp, V, Pp, Mp, (int)Pp, Mp);                // V = Lu^-1 Kuf          (layers.py:245)
-    g.a_tri = 1;
-    RC(gemm(c, g, false));
-    g = gargs(w.LinvT, Mp, V, Pp, A, Pp, Mp, (int)Pp, Mp);               // A = Lu^-T V            (layers.py:247)
-    g.a_tri = 2;
-    RC(gemm(c, g, false));
-    g = gargs(w.RpT, Mp, A, Pp, T, Pp, Mp, (int)Pp, Mp);                 // T_d = q_sqrt_d^T A     (layers.py:257-271)
-    g.a_tri = 2; g.batch = D; g.sA = (long)Mp * Mp; g.sB = 0; g.sC = (long)Mp * Pp;
-    RC(gemm(c, g, false));
+    RC(aform_forward(c, w, K, V, A, T, Pp));
   }
   if (mean) {
     CAT(DGP_CAT_MOMENTS);
@@ -1934,31 +1944,18 @@ int svgp_from_k_run(dgp_ctx* c, int M, int D, long P, const double* Ku, const do
   CAT(DGP_CAT_OTHER);
   LAUNCH(upstream_ext_kernel, (unsigned)(Pp / 128), 128, 0, Gm, Gv, P, Pp, D, GvT, GmPad, gq, dKdiag);
   CAT(DGP_CAT_GEMM_BWD_DATA);
-  g = gargs(w.qmuP, 32, GmPad, 32, dA, Pp, Mp, (int)Pp, 32);          // dA' = q_mu Gm^T + sum_d R_d (2 Gv_d o T_d)
-  RC(gemm(c, g, true));
-  g = gargs(w.Rcat, (long)D * Mp, T, Pp, dA, Pp, Mp, (int)Pp, D * Mp);
-  g.a_tri = 1; g.kblocks = D; g.kblk = Mp; g.bscale = GvT; g.ld_bscale = Pp; g.bscale_mul = 2.0; g.beta = 1.0;
-  if (D == 1) g.kblocks = 1;
-  RC(gemm(c, g, false));
-  g = gargs(w.Kinv, Mp, dA, Pp, W, Pp, Mp, (int)Pp, Mp);               // W = Ku^-1 dA'
-  RC(gemm(c, g, false));
+  RC(aform_adjoint(c, w, T, GmPad, GvT, dA, W, Pp, nullptr));
   CAT(DGP_CAT_RBF_BWD);
   LAUNCH(kbar_ext_kernel, (unsigned)(((size_t)M * Pp + 255) / 256), 256, 0, W, A, gq, M, P, Pp, dKuf);
   CAT(DGP_CAT_GEMM_BWD_PARAM);
   GemmArgs pg[3];
-  const bool pnt[3] = {true, true, false};
-  pg[0] = gargs(W, Pp, A, Pp, w.dKu, Mp, Mp, Mp, (int)Pp);             // dKu (data part) = -Wg A^T
-  pg[0].alpha = -1.0;
-  pg[1] = gargs(A, Pp, T, Pp, w.dR, Mp, Mp, Mp, (int)Pp);              // dq_sqrt_d (data part) = tril(A diag(2 Gv_d) T_d^T)
-  pg[1].alpha = 2.0; pg[1].batch = D; pg[1].sA = 0; pg[1].sB = (long)Mp * Pp; pg[1].sC = (long)Mp * Mp; pg[1].c_lower = 1;
-  pg[1].kscale = GvT; pg[1].sScale = Pp;
-  pg[2] = gargs(A, Pp, GmPad, 32, w.dqmu, 32, Mp, 32, (int)Pp);        // dq_mu (data part) = A Gm
+  aform_param_args(w, W, A, T, GvT, GmPad, Pp, 0.0, pg);
   CK(cudaMemsetAsync(w.dR, 0, (size_t)D * Mp * Mp * sizeof(double), c->stream));   // c_lower leaves the upper tiles unwritten
   for (int i = 0; i < 3; ++i) {
-    pg[i].splitk = pick_splitk(c, pg[i], pnt[i]);
+    pg[i].splitk = pick_splitk(c, pg[i], kAformParamNT[i]);
     if (pg[i].splitk > 1 && (size_t)pg[i].splitk * pg[i].batch * pg[i].M * pg[i].N > partcap) pg[i].splitk = 1;
     pg[i].part = part;
-    RC(gemm(c, pg[i], pnt[i]));
+    RC(gemm(c, pg[i], kAformParamNT[i]));
   }
   // ---- KL adjoint (weighted by gkl: the caller's d loss / d kl) and unpadding ----
   CAT(DGP_CAT_PREP);
@@ -2050,13 +2047,10 @@ int dgp_svgp_from_k(dgp_ctx* c, int M, int D_out, int64_t P, const double* Ku, c
                     const double* q_mu, const double* q_sqrt, double* mean, double* var, double* kl) {
   if (!c || !Ku || !Kuf || !Kdiag || !q_mu || !q_sqrt || !mean || !var || M < 1 || D_out < 1 || D_out > kMaxD || P < 1) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  c->dry = true; c->used = 0;
-  int rc = svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr);
+  return planned(c, [&] {
+    return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr,
+                           nullptr, nullptr);
+  });
 }
 
 int dgp_svgp_from_k_grad(dgp_ctx* c, int M, int D_out, int64_t P, const double* Ku, const double* Kuf, const double* Kdiag,
@@ -2065,30 +2059,22 @@ int dgp_svgp_from_k_grad(dgp_ctx* c, int M, int D_out, int64_t P, const double* 
   if (!c || !Ku || !Kuf || !Kdiag || !q_mu || !q_sqrt || !Gm || !Gv || !dKu || !dKuf || !dKdiag || !dq_mu || !dq_sqrt || M < 1 ||
       D_out < 1 || D_out > kMaxD || P < 1) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  c->dry = true; c->used = 0;
-  int rc = svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu, dq_sqrt);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu, dq_sqrt);
+  return planned(c, [&] {
+    return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu,
+                           dq_sqrt);
+  });
 }
 
 int64_t dgp_svgp_prep_cache_bytes(dgp_ctx* c, int M, int D_out) {
   if (!c || M < 1 || D_out < 1 || D_out > kMaxD) return -1;
-  dgp_layer_desc d;
-  memset(&d, 0, sizeof(d));
-  d.D_in = 1; d.D_out = D_out; d.M = M;
-  static const double unread = 0.0;      // the dry pass only lays the arena out: no pointer of the descriptor is dereferenced
-  d.Z = &unread; d.lengthscales = &unread; d.variance = &unread; d.q_mu = &unread; d.q_sqrt = &unread;
-  dgp_model_desc model{1, &d, nullptr};
+  static const double unread = 0.0;      // the dry pass only lays the arena out: no pointer it is given is dereferenced
   std::vector<LayerWs> lw;
-  const bool fused_saved = c->use_fused, dry_saved = c->dry;
+  const bool dry_saved = c->dry;
   const size_t used_saved = c->used;
-  c->use_fused = false; c->dry = true; c->used = 0;
-  int rc = prep_layers(c, &model, lw, PREP_GRAD, false, false, nullptr);
+  c->dry = true; c->used = 0;
+  const int rc = svgp_prep(c, M, D_out, &unread, &unread, &unread, PREP_GRAD, lw);
   const size_t bytes = c->used;
-  c->use_fused = fused_saved; c->dry = dry_saved; c->used = used_saved;
+  c->dry = dry_saved; c->used = used_saved;
   return rc == DGP_OK ? (int64_t)bytes : -1;
 }
 
@@ -2103,15 +2089,10 @@ int dgp_svgp_from_k_cached(dgp_ctx* c, int M, int D_out, int64_t P, const double
   if (!c || !Ku || !Kuf || !Kdiag || !q_mu || !q_sqrt || !mean || !var || !cache || cache_bytes < 1 || M < 1 || D_out < 1 ||
       D_out > kMaxD || P < 1) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  c->dry = true; c->used = 0;
-  int rc = svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                           cache, (size_t)cache_bytes, load != 0, stash);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                         cache, (size_t)cache_bytes, load != 0, stash);
+  return planned(c, [&] {
+    return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, mean, var, kl, nullptr, nullptr, 0.0, nullptr, nullptr, nullptr,
+                           nullptr, nullptr, cache, (size_t)cache_bytes, load != 0, stash);
+  });
 }
 
 int dgp_svgp_from_k_grad_cached(dgp_ctx* c, int M, int D_out, int64_t P, const double* Ku, const double* Kuf, const double* Kdiag,
@@ -2121,16 +2102,10 @@ int dgp_svgp_from_k_grad_cached(dgp_ctx* c, int M, int D_out, int64_t P, const d
   if (!c || !Ku || !Kuf || !Kdiag || !q_mu || !q_sqrt || !Gm || !Gv || !dKu || !dKuf || !dKdiag || !dq_mu || !dq_sqrt || !cache ||
       cache_bytes < 1 || M < 1 || D_out < 1 || D_out > kMaxD || P < 1) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  double* cc = const_cast<double*>(cache);
-  c->dry = true; c->used = 0;
-  int rc = svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu, dq_sqrt,
-                           cc, (size_t)cache_bytes, true, const_cast<double*>(stash));
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu, dq_sqrt,
-                         cc, (size_t)cache_bytes, true, const_cast<double*>(stash));
+  return planned(c, [&] {
+    return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu,
+                           dq_sqrt, const_cast<double*>(cache), (size_t)cache_bytes, true, const_cast<double*>(stash));
+  });
 }
 
 int64_t dgp_grad_size(const dgp_model_desc* model) {
@@ -2306,12 +2281,8 @@ int natgrad_outs(dgp_ctx* c, const std::vector<NatOut>& outs, long off, int maxM
     RC(gemm(c, g, false));
   }
   LAUNCH(natgrad_b_kernel, dim3(gx, (unsigned)nout), 256, 0, douts, T, gamma, Bf);
-  if (!c->chol_configured) {
-    CK(cudaFuncSetAttribute(chol_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_smem_bytes(768)));
-    c->chol_configured = true;
-  }
+  RC(chol_smem_optin(c));
   LAUNCH(chol_inv_kernel, nout, kCholThreads, chol_smem_bytes(maxMp), dargs);
-  CK(cudaFuncSetAttribute(tri_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tri_inv_smem_bytes(768)));
   LAUNCH(tri_inv_kernel, dim3((unsigned)(maxMp / 32), (unsigned)nout), 256, tri_inv_smem_bytes(maxMp), dargs, dinv, dinvT);
   LAUNCH(natgrad_flip_kernel, dim3(gx, (unsigned)nout), 256, 0, douts, LinvT, UinvT);
   for (int i = 0; i < nout; ++i) {   // C = R U^-T (lower x lower)
@@ -2323,35 +2294,19 @@ int natgrad_outs(dgp_ctx* c, const std::vector<NatOut>& outs, long off, int maxM
   LAUNCH(natgrad_finalize_kernel, nout, 256, 2 * (size_t)maxM * sizeof(double), douts, Cm, gamma, c->d_info);
   return DGP_OK;
 }
-
-int natgrad_planned(dgp_ctx* c, const dgp_model_desc* model, const int* layer_ids, int n_layers, double gamma, const double* grad_flat) {
-  c->dry = true; c->used = 0;
-  int rc = natgrad_run(c, model, layer_ids, n_layers, gamma, grad_flat);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return natgrad_run(c, model, layer_ids, n_layers, gamma, grad_flat);
-}
 }  // namespace
 
 int dgp_natgrad_step(dgp_ctx* c, const dgp_model_desc* model, const int* layer_ids, int n_layers, double gamma,
                      const double* grad_flat) {
   if (!c || !model || !layer_ids || n_layers < 0 || !grad_flat) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  return natgrad_planned(c, model, layer_ids, n_layers, gamma, grad_flat);
+  return planned(c, [&] { return natgrad_run(c, model, layer_ids, n_layers, gamma, grad_flat); });
 }
 
 int dgp_natgrad_pairs(dgp_ctx* c, const dgp_nat_pair* pairs, int n_pairs, double gamma) {
   if (!c || !pairs || n_pairs < 0) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  c->dry = true; c->used = 0;
-  int rc = natgrad_pairs_run(c, pairs, n_pairs, gamma);
-  c->dry = false;
-  if (rc != DGP_OK) return rc;
-  RC(ensure_ws(c, c->used));
-  c->used = 0;
-  return natgrad_pairs_run(c, pairs, n_pairs, gamma);
+  return planned(c, [&] { return natgrad_pairs_run(c, pairs, n_pairs, gamma); });
 }
 
 int dgp_train_nat_adam(dgp_ctx* c, const dgp_model_desc* model, const double* X, const double* Y, int64_t N, int64_t S, double scale,
@@ -2370,7 +2325,7 @@ int dgp_train_nat_adam(dgp_ctx* c, const dgp_model_desc* model, const double* X,
     if (have_adam) RC(adam_launch(c, tab, out_flat, m_state, v_state, t0 + k, lr, beta1, beta2, epsilon, elbo_trace ? elbo_trace + k : nullptr));
     else if (elbo_trace) LAUNCH(scale_copy_diff_kernel, 1, 32, 0, out_flat, elbo_trace + k);
     RC(dgp_elbo_grad(c, model, X, Y, N, S, scale, kl_weight, nullptr, seed0 + (uint64_t)(2 * k + 1) * seed_stride, n_offset, 1, out_flat));
-    RC(natgrad_planned(c, model, nat_layers, n_nat, gamma, out_flat));
+    RC(planned(c, [&] { return natgrad_run(c, model, nat_layers, n_nat, gamma, out_flat); }));
   }
   return DGP_OK;
 }
@@ -2437,10 +2392,7 @@ int dgp_ei(dgp_ctx* c, const dgp_model_desc* model, const double* X, int64_t N, 
 
 int dgp_ei_grad(dgp_ctx* c, const dgp_model_desc* model, const double* X, int64_t N, int64_t S, const double* const* zs_host,
                 uint64_t seed, int64_t n_offset, double y_min, double* neg_ei, double* d_neg_ei_dX) {
-  if (!c || !model || !X || !neg_ei || !d_neg_ei_dX) return DGP_ERR_ARG;
-  RunOpts o;
-  o.io.zs = zs_host; o.ei = neg_ei; o.y_min = y_min; o.ei_analytic = 1; o.dx = d_neg_ei_dX;
-  return run_model_planned(c, model, X, N, S, seed, n_offset, o);
+  return dgp_acq_grad(c, model, 0, X, N, S, zs_host, seed, n_offset, y_min, neg_ei, d_neg_ei_dX);
 }
 
 int dgp_acq_grad(dgp_ctx* c, const dgp_model_desc* model, int kind, const double* X, int64_t N, int64_t S,

@@ -11,7 +11,6 @@
 //   splitk > 1: K is cut into splitk chunks, partial tiles go to `part` and are summed in a fixed order
 //               (deterministic, no atomics) by gemm_splitk_reduce.
 #pragma once
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -390,9 +389,7 @@ inline int gemm_ctas_per_sm() {
 // NT products on 64x64 tiles (the contractions over the point-samples) run 32-deep k-tiles: half the barriers and loop
 // bookkeeping per flop (measured -4% on the parameter adjoints; the short-K NN products are faster with 16)
 inline bool gemm_small_bk32(const GemmArgs& g, bool nt) {
-  if (!nt) return false;
-  static const bool enabled = getenv("DGP_B200_GEMM_BK16") == nullptr;
-  if (!enabled || g.K % 32) return false;
+  if (!nt || g.K % 32) return false;
   if (g.kblocks > 1 && g.kblk % 32) return false;
   if (g.splitk > 1 && ((g.K / 32 + g.splitk - 1) / g.splitk) < 1) return false;
   return true;
@@ -400,8 +397,7 @@ inline bool gemm_small_bk32(const GemmArgs& g, bool nt) {
 
 // lower-only contraction over the point-samples on 64 x 64 x 32 tiles: strictly-lower and diagonal tiles as two launches (TSEL)
 inline bool gemm_split_diag(const GemmArgs& g, bool nt) {
-  static const bool enabled = getenv("DGP_B200_GEMM_ONE_LAUNCH") == nullptr;
-  return enabled && nt && g.c_lower && g.a_tri == 0 && g.kblocks <= 1 && g.M == g.N && g.M > 64 && g.K % 32 == 0 &&
+  return nt && g.c_lower && g.a_tri == 0 && g.kblocks <= 1 && g.M == g.N && g.M > 64 && g.K % 32 == 0 &&
          !((g.M % 128 == 0) && (g.N % 128 == 0) && ((long)g.M * g.N * g.batch >= 128L * 128 * 64));
 }
 
