@@ -89,6 +89,7 @@ _SIG = {
                                  _vp, _vp, _i64, _i64, _d, _d, _d, _d, _vp, _vp]),
     "dgp_comp_K": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp]),
     "dgp_comp_Kdiag": (C.c_int, [_vp, _vp, _vp, _i64, _vp]),
+    "dgp_comp_K_blocks": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _vp]),
     "dgp_comp_K_grad": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp]),
     "dgp_comp_Kdiag_grad": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "dgp_svgp_from_k": (C.c_int, [_vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -97,6 +98,7 @@ _SIG = {
     "dgp_svgp_stash_bytes": (_i64, [_i, _i, _i64]),
     "dgp_svgp_from_k_cached": (C.c_int, [_vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _vp]),
     "dgp_svgp_from_k_grad_cached": (C.c_int, [_vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "dgp_svgp_from_k_full_cov": (C.c_int, [_vp, _i, _i, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _d, _vp, _vp, _vp]),
     "dgp_comm_unique_id": (C.c_int, [_vp]),
     "dgp_comm_init": (C.c_int, [_vp, _i, _i, _vp]),
     "dgp_allreduce_grads": (C.c_int, [_vp, _vp, _i64]),

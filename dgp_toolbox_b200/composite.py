@@ -286,6 +286,45 @@ class SVGPFromK(torch.autograd.Function):
         return dKu, dKuf, dKdiag, dq_mu, dq_sqrt, None
 
 
+def _no_adjoint(name, tensors):
+    if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors):
+        raise NotImplementedError(f"{name}: the full_cov=True path has no adjoint; call it on tensors that do not require grad")
+
+
+def comp_K_blocks(roles, X, *theta):
+    """kern.K(X_b, X_b) [B, N, N] for X [B, N, D] (White on each block's diagonal) through dgp_comp_K_blocks: one launch for all
+    blocks. Forward only."""
+    _no_adjoint("comp_K_blocks", (X,) + theta)
+    th = {r: (None if t is None else t.detach().contiguous()) for r, t in zip(ROLE_PARAMS, theta)}
+    X = X.detach().contiguous()
+    B, N = X.shape[0], X.shape[1]
+    out = torch.empty((B, N, N), dtype=torch.float64, device=X.device)
+    d = _desc(roles, th)
+    _lib.get_context(X.device).call("dgp_comp_K_blocks", C.byref(d), _lib.ptr(X), B, N, _lib.ptr(out))
+    return out
+
+
+def svgp_from_k_full_cov(Ku, Kuf, Kff, q_mu, q_sqrt, z, jitter):
+    """SVGP_Layer.conditional_ND(full_cov=True) per sample + reparameterize(full_cov=True) (utils/layers.py:76-80,264-268,276;
+    utils/utils.py:43-52) on supplied Ku = Kuu + jitter I [M, M], Kuf [M, S*N] (column s*N + n), Kff [1 or S, N, N], draws z
+    [S, N, D_out] through dgp_svgp_from_k_full_cov -> (F [S, N, D_out], mean [S, N, D_out], cov [S, N, N, D_out]). Forward only:
+    raises NotImplementedError when an input requires grad."""
+    _no_adjoint("svgp_from_k_full_cov", (Ku, Kuf, Kff, q_mu, q_sqrt, z))
+    Ku, Kuf, Kff, q_mu, q_sqrt, z = [t.detach().contiguous() for t in (Ku, Kuf, Kff, q_mu, q_sqrt, z)]
+    S, N, D = z.shape
+    M = Ku.shape[0]
+    if Kuf.shape != (M, S * N) or Kff.shape[1:] != (N, N) or q_mu.shape != (M, D):
+        raise ValueError(f"svgp_from_k_full_cov: shapes Ku {tuple(Ku.shape)}, Kuf {tuple(Kuf.shape)}, Kff {tuple(Kff.shape)}, "
+                         f"q_mu {tuple(q_mu.shape)}, z {tuple(z.shape)} do not fit together")
+    mean = torch.empty((S, N, D), dtype=torch.float64, device=Ku.device)
+    cov = torch.empty((S, N, N, D), dtype=torch.float64, device=Ku.device)
+    F = torch.empty_like(mean)
+    _lib.get_context(Ku.device).call("dgp_svgp_from_k_full_cov", M, D, N, S, _lib.ptr(Ku), _lib.ptr(Kuf), _lib.ptr(Kff), Kff.shape[0],
+                                     _lib.ptr(q_mu), _lib.ptr(q_sqrt), _lib.ptr(z), float(jitter), _lib.ptr(mean), _lib.ptr(cov),
+                                     _lib.ptr(F))
+    return F, mean, cov
+
+
 class CompositeKernelEval:
     """K / K_diag of a lowered kernel on leaf tensors `th` (dict role -> tensor): differentiable through the library's adjoints."""
 
@@ -302,3 +341,7 @@ class CompositeKernelEval:
 
     def K_diag(self, X, values=None):
         return CompKdiag.apply(self.roles, X, *self.leaves(values or {}))
+
+    def K_blocks(self, X, values=None):
+        """K(X_b, X_b) [B, N, N] for X [B, N, D]; forward only (the full_cov=True path)."""
+        return comp_K_blocks(self.roles, X, *self.leaves(values or {}))

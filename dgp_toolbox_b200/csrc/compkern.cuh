@@ -51,6 +51,21 @@ __global__ void compk_K_kernel(CompK k, const double* __restrict__ X, long P, co
   K[idx] = v;
 }
 
+// K [B][N][N] = K(X_b, X_b) for the B blocks of X [B][N][D], White on each block's diagonal; grid (ceil(N^2 / 256), <= 65535),
+// the y index walks the blocks
+__global__ void compk_K_blocks_kernel(CompK k, const double* __restrict__ X, long B, long N, double* __restrict__ K) {
+  const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= N * N) return;
+  const long i = idx / N, j = idx % N;
+  for (long b = blockIdx.y; b < B; b += gridDim.y) {
+    const double* Xb = X + b * N * k.D;
+    CompParts q;
+    double v = compk_eval(k, Xb + i * k.D, Xb + j * k.D, q);
+    if (i == j && k.white_var) v += k.white_var[0];
+    K[b * N * N + idx] = v;
+  }
+}
+
 __global__ void compk_Kdiag_kernel(CompK k, const double* __restrict__ X, long P, double* __restrict__ out) {
   const long p = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= P) return;

@@ -1451,13 +1451,13 @@ int run_model_planned(dgp_ctx* c, const dgp_model_desc* model, const double* X, 
   return planned(c, [&] { return run_model(c, model, X, N, S, seed, n_offset, o); });
 }
 
-int check_chol(dgp_ctx* c) {
+int check_chol(dgp_ctx* c, const char* what = nullptr) {
   int info = 0;
   CK(cudaMemcpyAsync(&info, c->d_info, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   if (info) {
     CK(cudaMemsetAsync(c->d_info, 0, sizeof(int), c->stream));   // reported once; later steps start clean
-    c->err = "Kuu + jitter I is not positive definite (Cholesky pivot <= 0); parameter updates were suspended from that step on";
+    c->err = what ? what : "Kuu + jitter I is not positive definite (Cholesky pivot <= 0); parameter updates were suspended from that step on";
     return DGP_ERR_NUMERIC;
   }
   return DGP_OK;
@@ -1993,6 +1993,17 @@ int dgp_comp_Kdiag(dgp_ctx* c, const dgp_comp_kernel* k, const double* X, int64_
   return DGP_OK;
 }
 
+int dgp_comp_K_blocks(dgp_ctx* c, const dgp_comp_kernel* k, const double* X, int64_t B, int64_t N, double* K_out) {
+  if (!c || !X || !K_out || B < 1 || N < 1) return DGP_ERR_ARG;
+  RC(comp_check(c, k));
+  CK(cudaSetDevice(c->device));
+  const long nn = (long)N * N;
+  CAT(DGP_CAT_KUF);
+  LAUNCH(compk_K_blocks_kernel, dim3((unsigned)((nn + 255) / 256), (unsigned)(B < 65535 ? B : 65535)), 256, 0, comp_view(k), X, (long)B,
+         (long)N, K_out);
+  return DGP_OK;
+}
+
 int dgp_comp_K_grad(dgp_ctx* c, const dgp_comp_kernel* k, const double* X, int64_t P, const double* X2, int64_t P2,
                     const double* Kbar, double* dX, double* dX2, double* dtheta) {
   if (!c || !X || !Kbar || !dX || !dtheta || P < 1 || (X2 && (P2 < 1 || !dX2))) return DGP_ERR_ARG;
@@ -2106,6 +2117,76 @@ int dgp_svgp_from_k_grad_cached(dgp_ctx* c, int M, int D_out, int64_t P, const d
     return svgp_from_k_run(c, M, D_out, P, Ku, Kuf, Kdiag, q_mu, q_sqrt, nullptr, nullptr, nullptr, Gm, Gv, gkl, dKu, dKuf, dKdiag, dq_mu,
                            dq_sqrt, const_cast<double*>(cache), (size_t)cache_bytes, true, const_cast<double*>(stash));
   });
+}
+
+namespace {
+// full_cov=True on supplied matrices: the prep and the A-form planes of dgp_svgp_from_k over all S * N columns (so the mean is the
+// same computation), then, as run_full_cov does on its V-form planes, the S * D_out covariance blocks, their factors and the samples.
+int svgp_full_cov_run(dgp_ctx* c, int M, int D, long N, long S, const double* Ku, const double* Kuf, const double* Kff, long Kff_batch,
+                      const double* q_mu, const double* q_sqrt, const double* z, double jitter, double* mean, double* cov, double* F) {
+  std::vector<LayerWs> lw;
+  RC(svgp_prep(c, M, D, Ku, q_mu, q_sqrt, PREP_FWD, lw));
+  const LayerWs& w = lw[0];
+  const int Mp = w.Mp;
+  const long P = N * S, Pp = round_up(P, kTileP), Np = round_up(N, kTileM);
+  const size_t plane = (size_t)Mp * Pp, nblk = (size_t)S * D, blk = (size_t)Np * Np;
+  const bool blocks = cov || F;
+  const size_t need = (plane * (3 + (size_t)D) + (size_t)P * (D + 1) + (blocks ? 1 : 0) * nblk * blk + (F ? 1 : 0) * nblk * blk) * sizeof(double);
+  if (need + c->used > c->ws_limit) {
+    c->err = "dgp_svgp_from_k_full_cov: S * N too large for the workspace limit (dgp_set_workspace_limit); split the samples";
+    return DGP_ERR_UNSUPPORTED;
+  }
+  double* K = walloc(c, plane);
+  double* V = walloc(c, plane);
+  double* A = walloc(c, plane);
+  double* T = walloc(c, plane * D);
+  double* kzero = walloc(c, (size_t)P);           // K_diag of moments_ext_kernel: its variance is not used, the blocks carry it
+  double* vscr = walloc(c, (size_t)P * D);
+  double* cin = blocks ? walloc(c, nblk * blk) : nullptr;
+  double* Lf = F ? walloc(c, nblk * blk) : nullptr;
+  CholArgs* dargs = F ? reinterpret_cast<CholArgs*>(walloc(c, (sizeof(CholArgs) * nblk + 7) / 8)) : nullptr;
+  if (c->dry) return DGP_OK;
+  CAT(DGP_CAT_GEMM_FWD);
+  LAUNCH(pad_plane_kernel, (unsigned)((plane + 255) / 256), 256, 0, Kuf, M, Mp, P, Pp, K);
+  RC(aform_forward(c, w, K, V, A, T, Pp));
+  CAT(DGP_CAT_MOMENTS);
+  CK(cudaMemsetAsync(kzero, 0, (size_t)P * sizeof(double), c->stream));
+  LAUNCH(moments_ext_kernel, (unsigned)((P + 127) / 128), 128, 0, V, A, T, w.qmuP, kzero, M, Mp, D, P, Pp, mean, vscr);
+  if (!blocks) return DGP_OK;
+  FullCovArgs f;
+  memset(&f, 0, sizeof(f));
+  f.V = V; f.T = T; f.Mp = Mp; f.D = D; f.N = N; f.Np = Np; f.Pp = Pp; f.S = (int)S; f.jitter = jitter;
+  f.var_out = cov; f.chol_in = cin;
+  const unsigned nt = (unsigned)(Np / kFcTile);
+  LAUNCH(fullcov_ext_kernel, dim3(nt, nt, (unsigned)nblk), 256, 0, f, Kff, Kff_batch == 1 ? 0L : N * N);
+  if (!F) return DGP_OK;
+  std::vector<CholArgs> hargs(nblk);
+  for (size_t i = 0; i < nblk; ++i) hargs[i] = CholArgs{cin + i * blk, Lf + i * blk, nullptr, nullptr, (int)Np, c->d_info};
+  H2D(dargs, hargs.data(), sizeof(CholArgs) * nblk);
+  RC(chol_smem_optin(c));
+  LAUNCH(chol_inv_kernel, (unsigned)nblk, kCholThreads, chol_smem_bytes((int)Np), dargs);
+  LAUNCH(fullcov_sample_kernel, dim3((unsigned)((N + 127) / 128), (unsigned)nblk), 128, 0, Lf, mean, z, N, Np, D, (int)S, F, nullptr);
+  return DGP_OK;
+}
+}  // namespace
+
+int dgp_svgp_from_k_full_cov(dgp_ctx* c, int M, int D_out, int64_t N, int64_t S, const double* Ku, const double* Kuf,
+                             const double* Kff, int64_t Kff_batch, const double* q_mu, const double* q_sqrt, const double* z,
+                             double jitter, double* mean, double* cov, double* F) {
+  if (!c) return DGP_ERR_ARG;
+  if (!Ku || !Kuf || !Kff || !q_mu || !q_sqrt || !mean || M < 1 || D_out < 1 || D_out > kMaxD || N < 1 || S < 1) {
+    c->err = "dgp_svgp_from_k_full_cov: null input or output, or a size out of range (M >= 1, 1 <= D_out <= 32, N >= 1, S >= 1)";
+    return DGP_ERR_ARG;
+  }
+  if (round_up(N, kTileM) > 768) {
+    c->err = "dgp_svgp_from_k_full_cov: N > 768 is not supported (one CTA factorises an N x N block)"; return DGP_ERR_UNSUPPORTED;
+  }
+  if (Kff_batch != 1 && Kff_batch != S) { c->err = "dgp_svgp_from_k_full_cov: Kff_batch must be 1 (one shared block) or S"; return DGP_ERR_ARG; }
+  if (F && !z) { c->err = "dgp_svgp_from_k_full_cov: F needs the draws z"; return DGP_ERR_ARG; }
+  if (S * D_out > 65535) { c->err = "dgp_svgp_from_k_full_cov: S * D_out > 65535 covariance blocks"; return DGP_ERR_UNSUPPORTED; }
+  CK(cudaSetDevice(c->device));
+  RC(planned(c, [&] { return svgp_full_cov_run(c, M, D_out, N, S, Ku, Kuf, Kff, Kff_batch, q_mu, q_sqrt, z, jitter, mean, cov, F); }));
+  return check_chol(c, "dgp_svgp_from_k_full_cov: Ku or a block cov + jitter I is not positive definite (Cholesky pivot <= 0)");
 }
 
 int64_t dgp_grad_size(const dgp_model_desc* model) {

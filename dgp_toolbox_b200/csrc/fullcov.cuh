@@ -4,6 +4,8 @@
 // In the V-form planes the forward kernel stashes (V = Lu^-1 Kuf [Mp][Pp], T_d = C_d V [D][Mp][Pp], columns p = s N + n):
 //   cov_{s,d}[n][n'] = k(x_sn, x_sn') - sum_m V[m][sN+n] V[m][sN+n'] + sum_m T_d[m][sN+n] T_d[m][sN+n'].
 // The N x N blocks are small (N <= 768: one CTA factorises a block), so the Gram products run as shared-memory tiled FP64 FMAs.
+// The supplied-matrix path (dgp_svgp_from_k_full_cov) builds the same Gram on its A-form planes (V = Lu^-1 Kuf, T_d = q_sqrt_d^T A,
+// so T_d^T T_d = A^T q_sqrt_d q_sqrt_d^T A and V^T V = A^T Ku A) with the k term read from the caller's Kff: fullcov_ext_kernel.
 #pragma once
 #include "common.cuh"
 
@@ -21,8 +23,10 @@ struct FullCovArgs {
 
 constexpr int kFcTile = 32;
 
-// grid: (Np / 32, Np / 32, S * D); block 32 x 8
-__global__ void __launch_bounds__(256) fullcov_kernel(FullCovArgs a) {
+// One 32 x 32 tile of a covariance block. The K term is the layer's stationary kernel on the input rows, or (EXT) the caller's
+// block Kff[s * kff_stride + i * N + j] (the supplied-matrix path: dgp_svgp_from_k_full_cov).
+template <bool EXT>
+__device__ __forceinline__ void fullcov_tile(const FullCovArgs& a, const double* __restrict__ Kff, long kff_stride) {
   __shared__ double vi[kFcTile][kFcTile + 1], vj[kFcTile][kFcTile + 1], ti[kFcTile][kFcTile + 1], tj[kFcTile][kFcTile + 1];
   const int s = blockIdx.z / a.D, d = blockIdx.z % a.D;
   const int i0 = blockIdx.y * kFcTile, j0 = blockIdx.x * kFcTile;
@@ -58,19 +62,33 @@ __global__ void __launch_bounds__(256) fullcov_kernel(FullCovArgs a) {
     const int i = i0 + ty + 8 * u;
     double out_pad = (i == j) ? 1.0 : 0.0;
     if (i < a.N && j < a.N) {
-      const double* xi = a.Xin + ((c0 + i) % a.xmod) * a.D_in;
-      const double* xj = a.Xin + ((c0 + j) % a.xmod) * a.D_in;
-      double r2 = 0.0;
-      for (int q = 0; q < a.D_in; ++q) {
-        const double t = (xi[q] - xj[q]) / a.ls[q];
-        r2 = fma(t, t, r2);
+      double k;
+      if (EXT) {
+        k = Kff[(long)s * kff_stride + (long)i * a.N + j];
+      } else {
+        const double* xi = a.Xin + ((c0 + i) % a.xmod) * a.D_in;
+        const double* xj = a.Xin + ((c0 + j) % a.xmod) * a.D_in;
+        double r2 = 0.0;
+        for (int q = 0; q < a.D_in; ++q) {
+          const double t = (xi[q] - xj[q]) / a.ls[q];
+          r2 = fma(t, t, r2);
+        }
+        k = kernel_value(a.kind, r2, a.var[0]);
       }
-      const double cov = kernel_value(a.kind, r2, a.var[0]) + acc[u];
+      const double cov = k + acc[u];
       if (a.var_out) a.var_out[(((long)s * a.N + i) * a.N + j) * a.D + d] = cov;
       out_pad = cov + (i == j ? a.jitter : 0.0);
     }
     if (i < a.Np && j < a.Np) a.chol_in[((long)blockIdx.z * a.Np + i) * a.Np + j] = out_pad;
   }
+}
+
+// grid: (Np / 32, Np / 32, S * D); block 32 x 8
+__global__ void __launch_bounds__(256) fullcov_kernel(FullCovArgs a) { fullcov_tile<false>(a, nullptr, 0); }
+
+// the same with the K term read from Kff [.][N][N]: kff_stride = N * N (one block per sample) or 0 (one block shared by all)
+__global__ void __launch_bounds__(256) fullcov_ext_kernel(FullCovArgs a, const double* __restrict__ Kff, long kff_stride) {
+  fullcov_tile<true>(a, Kff, kff_stride);
 }
 
 // F[s][n][d] = mean[s][n][d] + sum_{n' <= n} L_{s,d}[n][n'] z[s][n'][d]        (utils/utils.py:50)

@@ -17,7 +17,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..composite import EVAL_CACHE, RBF, CompositeKernelEval, LinearKernel, PrepCache, SVGPFromK, White, stash_budget_bytes
+from ..composite import (EVAL_CACHE, RBF, CompositeKernelEval, LinearKernel, PrepCache, SVGPFromK, White, stash_budget_bytes,
+                         svgp_from_k_full_cov)
 from ..gpflow_shim import DEFAULT_JITTER, Gaussian, Parameter, _Module, set_trainable
 
 
@@ -93,8 +94,11 @@ class MFLayer(_Module):
         return SVGPFromK.apply(ent["Ku"], Kuf, Kdiag, values.get(self.q_mu, self.q_mu.value), values.get(self.q_sqrt, self.q_sqrt.value),
                                ent["prep"])
 
-    def sample_from_conditional(self, X, z=None, values=None, draw=None):
-        """utils/layers.py:87-130, full_cov = False: X [S, N, D] -> samples, mean, var [S, N, D_out]."""
+    def sample_from_conditional(self, X, z=None, values=None, draw=None, full_cov=False, shared_input=False):
+        """utils/layers.py:87-130: X [S, N, D] -> samples, mean [S, N, D_out], var [S, N, D_out] (full_cov=True: [S, N, N, D_out]).
+        shared_input: every sample's input is X[0] (the first application of a chain), so K(X_s, X_s) is one shared block."""
+        if full_cov:
+            return self._sample_full_cov(X, z, values, draw, shared_input)
         S, N, D = X.shape
         mean, var, _ = self.conditional_ND(X.reshape(S * N, D), values)
         mean, var = mean.reshape(S, N, self.num_outputs), var.reshape(S, N, self.num_outputs)
@@ -102,11 +106,37 @@ class MFLayer(_Module):
             z = (draw or _default_draw(self.device))((S, N, self.num_outputs))
         return mean + z * torch.sqrt(var + DEFAULT_JITTER), mean, var
 
+    def _sample_full_cov(self, X, z, values, draw, shared_input):
+        """conditional_SND(full_cov=True) + reparameterize(full_cov=True) (utils/layers.py:76-80,264-268,276; utils/utils.py:43-52):
+        per sample the N x N covariance and a correlated draw, one dgp_svgp_from_k_full_cov call. Forward only. The draws are one
+        `draw((S, N, D_out))`, as on the diagonal path, so seeds and recorded draws line up across the two modes."""
+        values = values or {}
+        S, N, D = X.shape
+        if D < self.D:
+            raise ValueError(f"the layer's kernel addresses {self.D} input columns, got {D}")
+        Xk = X[:, :, :self.D]
+        Z = self.Zfull(values)
+        Ku = self.eval.K(Z, None, values) + DEFAULT_JITTER * torch.eye(self.num_inducing, dtype=torch.float64, device=X.device)
+        Kuf = self.eval.K(Z, Xk.reshape(S * N, self.D).contiguous(), values)
+        Kff = self.eval.K_blocks(Xk[:1] if shared_input else Xk, values)
+        if z is None:
+            z = (draw or _default_draw(self.device))((S, N, self.num_outputs))
+        z = z.expand(S, N, self.num_outputs)
+        return svgp_from_k_full_cov(Ku, Kuf, Kff, values.get(self.q_mu, self.q_mu.value), values.get(self.q_sqrt, self.q_sqrt.value), z,
+                                    DEFAULT_JITTER)
+
     def KL(self, values=None):
         """utils/layers.py:280-308 (one dummy point: the KL needs Ku and q only)."""
         values = values or {}
         Z = self.Zfull(values)
         return self.conditional_ND(Z[:1].detach(), values)[2]
+
+
+def check_full_cov_inputs(X, values):
+    """The full_cov=True path has no adjoint: refuse inputs that ask for one rather than return a silently detached result."""
+    leaves = [X] + [v for v in (values or {}).values() if isinstance(v, torch.Tensor)]
+    if any(isinstance(t, torch.Tensor) and t.requires_grad for t in leaves):
+        raise NotImplementedError("full_cov=True has no adjoint: X and the tensors in `values` must not require grad")
 
 
 def _chol(K):
@@ -188,9 +218,10 @@ class DGP_Base(_Module):
         return self.layers[0].device
 
     def propagate(self, X, full_cov=False, S=1, zs=None, values=None):
-        """MF_DGP.py:98-132: layer l >= 1 sees the input augmented with the previous layer's sample."""
+        """MF_DGP.py:98-132: layer l >= 1 sees the input augmented with the previous layer's sample. full_cov=True: Fvars[l] is
+        [S, N, N, D_l] and the samples are correlated over the N points (forward only, N <= 768)."""
         if full_cov:
-            raise NotImplementedError("full_cov=True is not available for the multi-fidelity layers")
+            check_full_cov_inputs(X, values)
         X = _lib.as_device(X, self.device)
         sX = X[None].expand(S, -1, -1)
         Fs, Fmeans, Fvars = [], [], []
@@ -199,12 +230,12 @@ class DGP_Base(_Module):
         for i, (layer, z) in enumerate(zip(self.layers, zs)):
             inp = F if i == 0 else torch.cat([sX, F], 2)
             z = None if z is None else _lib.as_device(z, self.device)
-            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=z, values=values, draw=self.draw)
+            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=z, values=values, draw=self.draw, full_cov=full_cov, shared_input=i == 0)
             Fs.append(F); Fmeans.append(Fmean); Fvars.append(Fvar)
         return Fs, Fmeans, Fvars
 
     def predict_f(self, X, full_cov=False, S=1, fidelity=None, values=None):
-        """MF_DGP.py:134-149."""
+        """MF_DGP.py:134-149 (full_cov=True: the variance is [S, N, N, D])."""
         _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values)
         f = -1 if fidelity is None else fidelity
         return Fmeans[f], Fvars[f]
@@ -270,7 +301,8 @@ class DGP_Base(_Module):
             return self.propagate(Xnew, S=num_samples)
 
     def predict_y(self, Xnew, num_samples, full_cov=False):
-        """MF_DGP.py:238-240."""
+        """MF_DGP.py:238-240. `full_cov` is accepted and not passed on: this returns the diagonal moments whatever it is (whether
+        the reference passes it on is not pinned by a test of the reference's own code)."""
         with torch.no_grad():
             Fmean, Fvar = self.predict_f(Xnew, S=num_samples)
             return Fmean, Fvar + self.likelihood.likelihood.variance.value

@@ -11,7 +11,7 @@ import torch
 from .. import _lib
 from ..composite import EVAL_CACHE, RBF, LinearKernel, White
 from ..gpflow_shim import Gaussian, _Module, set_trainable
-from .MF_DGP import MFLayer, _Lik, _adam_step, sample
+from .MF_DGP import MFLayer, _Lik, _adam_step, check_full_cov_inputs, sample
 
 
 def sample_Z_right(layers, layers_red, Z, values=None, draw=None, num_samples=50):
@@ -62,9 +62,11 @@ class DGP_Base(_Module):
         return self.layers[0].device
 
     def propagate(self, X, full_cov=False, S=1, zs=None, ws=None, fidelity_dim=None, project=False, values=None):
-        """MF_DGP_EM.py:120-168: X lives in the input space of fidelity `fidelity_dim` (default: the highest)."""
+        """MF_DGP_EM.py:120-168: X lives in the input space of fidelity `fidelity_dim` (default: the highest). full_cov=True: the
+        variances (Hvars with project=True) are [S, N, N, D] and the samples are correlated over the N points (forward only,
+        N <= 768)."""
         if full_cov:
-            raise NotImplementedError("full_cov=True is not available for the multi-fidelity layers")
+            check_full_cov_inputs(X, values)
         X = _lib.as_device(X, self.device)
         sX = X[None].expand(S, -1, -1)
         L = len(self.layers_red)
@@ -73,19 +75,24 @@ class DGP_Base(_Module):
         ws = ws or [None] * L
         dev = lambda z: None if z is None else _lib.as_device(z, self.device)
         H, Hs, Hmeans, Hvars = sX, [sX], [], []
-        for layer_red, w in zip(self.layers_red[L - fidelity_dim:], ws[L - fidelity_dim:]):
-            H, Hmean, Hvar = layer_red.sample_from_conditional(H, z=dev(w), values=values, draw=self.draw)
+        # the first application of the chain sees X itself for every sample: the first projection layer, or layer 0 without one
+        for j, (layer_red, w) in enumerate(zip(self.layers_red[L - fidelity_dim:], ws[L - fidelity_dim:])):
+            H, Hmean, Hvar = layer_red.sample_from_conditional(H, z=dev(w), values=values, draw=self.draw, full_cov=full_cov,
+                                                               shared_input=j == 0)
             Hs.append(H); Hmeans.append(Hmean); Hvars.append(Hvar)
         if project:
             return Hs, Hmeans, Hvars
         Fs, Fmeans, Fvars = [], [], []
         for i, (layer, z) in enumerate(zip(self.layers[:fidelity_dim + 1], zs[:fidelity_dim + 1])):
             inp = Hs[-1] if i == 0 else torch.cat([Hs[-(i + 1)], F], 2)
-            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=dev(z), values=values, draw=self.draw)
+            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=dev(z), values=values, draw=self.draw, full_cov=full_cov,
+                                                           shared_input=i == 0 and len(Hs) == 1)
             Fs.append(F); Fmeans.append(Fmean); Fvars.append(Fvar)
         return Fs, Fmeans, Fvars
 
     def predict_f(self, X, full_cov=False, S=1, fidelity=None, fidelity_dim=None, values=None):
+        """`full_cov` is accepted and not passed on (so is `project`'s): both return the diagonal moments whatever it is. Whether the
+        reference passes it on is not pinned by a test of the reference's own code; propagate(full_cov=True) gives the covariances."""
         _, Fmeans, Fvars = self.propagate(X, S=S, fidelity_dim=fidelity_dim, values=values)
         f = -1 if fidelity is None else fidelity
         return Fmeans[f], Fvars[f]

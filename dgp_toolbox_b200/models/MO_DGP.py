@@ -71,19 +71,21 @@ class DGP_Base(_MF.DGP_Base):
         """MO_DGP.py:88-122 -> (Fs, Fmeans, Fvars), two entries each (objective 0, objective 1), [S, N, 1]. The chain starts from one
         N(0,1) column per point (shared by the S samples), runs layer 0, then alternates layers 1, 0, 1, 0 ... (2 loop applications;
         loop = 0: layer 1 once), reads objective 0 from the last application and objective 1 from one more application of layer 1.
-        `zs[k]`, when given, is reused by every application of layer k, as in the reference."""
+        `zs[k]`, when given, is reused by every application of layer k, as in the reference. full_cov=True: Fvars are [S, N, N, 1]
+        and the samples are correlated over the N points (forward only, N <= 768)."""
         if full_cov:
-            raise NotImplementedError("full_cov=True is not available for the composite-kernel layers")
+            _MF.check_full_cov_inputs(X, values)
         if not (isinstance(X, torch.Tensor) and X.requires_grad):      # a leaf the caller differentiates w.r.t. (EHVI_with_grad)
             X = _lib.as_device(X, self.device)
         sX = X[None].expand(S, -1, -1)
         zs = [None if z is None else _lib.as_device(z, self.device) for z in (zs or [None] * len(self.layers))]
 
-        def apply(k, F):
-            return self.layers[k].sample_from_conditional(torch.cat([sX, F], 2), z=zs[k], values=values, draw=self.draw)
+        def apply(k, F, shared=False):
+            return self.layers[k].sample_from_conditional(torch.cat([sX, F], 2), z=zs[k], values=values, draw=self.draw,
+                                                          full_cov=full_cov, shared_input=shared)
 
         F = _start_column(X.shape[0], self.device, self.draw)[None].expand(S, -1, -1)
-        F, Fmean, Fvar = apply(0, F)
+        F, Fmean, Fvar = apply(0, F, shared=True)      # [x, start column] is the same for every sample
         if self.loop == 0:
             F, Fmean, Fvar = apply(1, F)
         else:
@@ -95,7 +97,7 @@ class DGP_Base(_MF.DGP_Base):
         return Fs, Fmeans, Fvars
 
     def predict_f(self, X, full_cov=False, S=1, objective=None, values=None, fidelity=None):
-        """MO_DGP.py:124-138."""
+        """MO_DGP.py:124-138 (full_cov=True: the variance is [S, N, N, 1])."""
         objective = fidelity if objective is None else objective
         _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values)
         o = -1 if objective is None else objective

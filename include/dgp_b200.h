@@ -194,6 +194,10 @@ typedef struct {
  * SquaredExponential / Linear / White semantics with active_dims). */
 int dgp_comp_K(dgp_ctx* ctx, const dgp_comp_kernel* k, const double* X, int64_t P, const double* X2, int64_t P2, double* K_out);
 int dgp_comp_Kdiag(dgp_ctx* ctx, const dgp_comp_kernel* k, const double* X, int64_t P, double* out);
+/* kern.K(X_b, X_b) for B blocks of N rows: X [B, N, D] -> K_out [B, N, N], the White variance on each block's diagonal, exactly as
+ * dgp_comp_K with X2 = NULL gives for one block. One launch for all blocks: the K(X_s, X_s) of every sample of a layer application
+ * (each sample of a layer >= 1 has its own augmented input [x, f_{l-1,s}]). Same descriptor checks and argument errors as dgp_comp_K. */
+int dgp_comp_K_blocks(dgp_ctx* ctx, const dgp_comp_kernel* k, const double* X, int64_t B, int64_t N, double* K_out);
 /* Adjoints: given Kbar = d loss / d K [P, P2] -> dX [P, D], dX2 [P2, D] (NULL with X2 = NULL: dX then carries both roles) and
  * dtheta [DGP_COMP_THETA + (in_ard ? Da : 1)]; given g = d loss / d K_diag [P] -> dX, dtheta. Deterministic reductions. */
 int dgp_comp_K_grad(dgp_ctx* ctx, const dgp_comp_kernel* k, const double* X, int64_t P, const double* X2, int64_t P2,
@@ -227,6 +231,21 @@ int dgp_svgp_from_k_grad_cached(dgp_ctx* ctx, int M, int D_out, int64_t P, const
                                 const double* q_mu, const double* q_sqrt, const double* Gm, const double* Gv, double gkl,
                                 double* dKu, double* dKuf, double* dKdiag, double* dq_mu, double* dq_sqrt, const double* cache,
                                 int64_t cache_bytes, const double* stash);
+
+/* SVGP_Layer.conditional_ND(full_cov=True) per sample and reparameterize(full_cov=True) (utils/layers.py:76-80,264-268,276;
+ * utils/utils.py:43-52) on supplied matrices, white = False, no mean function (the MF / MO / EM layers). S samples of N points,
+ * column p = s * N + n:
+ *   Ku [M, M] = Kuu + jitter I, Kuf [M, S * N], Kff [Kff_batch, N, N] (Kff_batch = 1: one block shared by every sample, or S),
+ *   q_mu [M, D_out], q_sqrt [D_out, M, M]  ->
+ *   mean [S, N, D_out] (the mean dgp_svgp_from_k gives for the same Ku, Kuf, q);
+ *   cov  [S, N, N, D_out] = Kff_s + A_s^T (q_sqrt_d q_sqrt_d^T - Ku) A_s, A_s = Ku^-1 Kuf_s      (may be NULL);
+ *   F    [S, N, D_out]    = mean + chol(cov_sd + jitter I) z_sd                                   (may be NULL; F needs z [S, N, D_out]).
+ * N <= 768 (one CTA factorises an N x N block), S * D_out <= 65535 blocks; M and D_out as dgp_svgp_from_k. Every argument and the workspace limit are checked
+ * before the first launch. Forward only; factorises Ku itself (no prep cache). Synchronises; DGP_ERR_NUMERIC when Ku or a block
+ * cov_sd + jitter I is not positive definite. */
+int dgp_svgp_from_k_full_cov(dgp_ctx* ctx, int M, int D_out, int64_t N, int64_t S, const double* Ku, const double* Kuf,
+                             const double* Kff, int64_t Kff_batch, const double* q_mu, const double* q_sqrt, const double* z,
+                             double jitter, double* mean, double* cov, double* F);
 
 /* ---- multi-GPU (SURVEY §8b/e): one process (or thread) and one ctx per GPU. The minibatch's points are sharded over the ranks by
  * the caller; parameters, Kuu, its Cholesky and the KL term are replicated; the path's only exchange step is ONE sum-allreduce of the
