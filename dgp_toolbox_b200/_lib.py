@@ -110,6 +110,8 @@ _SIG = {
                                      _vp, _vp, _i64, _i64, _d, _d, _d, _d, C.POINTER(C.c_int), _i, _d, _vp, _vp]),
     "dgp_propagate_full_cov": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, C.POINTER(_vp),
                                          C.POINTER(_vp), C.POINTER(_vp)]),
+    "dgp_propagate_full_cov_snd": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, C.POINTER(_vp),
+                                             C.POINTER(_vp), C.POINTER(_vp)]),
     "dgp_e_log_p_y": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, _vp]),
     "dgp_predict_moments": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, _i,
                                       _vp, _vp]),

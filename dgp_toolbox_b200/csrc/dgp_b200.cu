@@ -1770,20 +1770,25 @@ int dgp_propagate(dgp_ctx* c, const dgp_model_desc* model, const double* X, int6
 
 namespace {
 // propagate(full_cov=True): per layer the fused conditional (V-form, stash on) gives mean, V and T_d for all S samples at once;
-// the S * D_out covariance blocks, their Cholesky factors and the correlated samples follow (fullcov.cuh).
-int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, long S, const double* const* zs_host,
-                 unsigned long long seed, long n_offset, double* const* Fs_host, double* const* Fmeans_host,
-                 double* const* Fvars_host) {
+// the S * D_out covariance blocks, their Cholesky factors and the correlated samples follow (fullcov.cuh). A layer the fused kernel
+// does not take (dgp_set_fused(0), or a shape no configuration fits) runs the unfused pipeline: its A-form planes V = Lu^-1 Kuf and
+// T_d = q_sqrt_d^T A give the same Gram (V^T V = A^T Ku A, T_d^T T_d = A^T q_sqrt_d q_sqrt_d^T A). x_per_sample: the first layer's
+// input is X [S][N][D_in] instead of X [N][D_in] shared by the samples.
+int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, bool x_per_sample, long N, long S,
+                 const double* const* zs_host, unsigned long long seed, long n_offset, double* const* Fs_host,
+                 double* const* Fmeans_host, double* const* Fvars_host) {
   RC(check_chain(c, model, N, S));
   const int nl = model->num_layers;
   const long Np = round_up(N, kTileM);
   if (Np > 768) { c->err = "full_cov=True: N > 768 is not supported (one CTA factorises an N x N block)"; return DGP_ERR_UNSUPPORTED; }
   std::vector<LayerWs> lw;
-  RC(prep_layers(c, model, lw, PREP_FWD, {c->use_fused, true}));   // the covariance blocks are built from the V-form planes
+  RC(prep_layers(c, model, lw, PREP_FWD, {c->use_fused, true}));   // fused layers: the covariance blocks come from the V-form planes
   const long P = N * S, Pp = round_up(P, kTileP);
   int maxD = 1;
+  bool any_unfused = false;
   for (int l = 0; l < nl; ++l) {
-    if (lw[l].fcfg < 0 || !lw[l].vform) { c->err = "full_cov=True needs a layer shape the fused conditional kernel supports"; return DGP_ERR_UNSUPPORTED; }
+    if (!moments_fit(c, lw[l])) return DGP_ERR_UNSUPPORTED;
+    if (lw[l].fcfg < 0) any_unfused = true;
     if (lw[l].D_out > maxD) maxD = lw[l].D_out;
   }
   std::vector<ChunkLayer> cls(nl);
@@ -1801,7 +1806,8 @@ int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long 
   double* cin = walloc(c, nblk * Np * Np);
   double* Lf = walloc(c, nblk * Np * Np);
   CholArgs* dargs = reinterpret_cast<CholArgs*>(walloc(c, (sizeof(CholArgs) * nblk + 7) / 8));
-  Temps tmp;
+  Temps tmp;   // unfused layers: Kuf in t0, V in t1 (A goes to planeV)
+  if (any_unfused) { tmp.t0 = walloc(c, (size_t)maxMp * Pp); tmp.t1 = walloc(c, (size_t)maxMp * Pp); }
   if (c->dry) return DGP_OK;
   std::vector<CholArgs> hargs(nblk);
   for (size_t i = 0; i < nblk; ++i) hargs[i] = CholArgs{cin + i * Np * Np, Lf + i * Np * Np, nullptr, nullptr, (int)Np, c->d_info};
@@ -1811,7 +1817,7 @@ int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long 
     const dgp_layer_desc& d = model->layers[l];
     const LayerWs& w = lw[l];
     ChunkLayer& cl = cls[l];
-    if (l == 0) { cl.Xin = X; cl.xmod = N; } else { cl.Xin = cls[l - 1].F; cl.xmod = P; }
+    if (l == 0) { cl.Xin = X; cl.xmod = x_per_sample ? P : N; } else { cl.Xin = cls[l - 1].F; cl.xmod = P; }
     cl.A = planeV; cl.T = planeT;
     ChunkIO io;   // means go straight to the caller; variances / samples are replaced by the full-covariance ones below
     std::vector<double*> fm(nl, nullptr);
@@ -1820,11 +1826,11 @@ int run_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long 
     CAT(DGP_CAT_MOMENTS);
     FullCovArgs f;
     memset(&f, 0, sizeof(f));
-    f.V = cl.A; f.T = cl.T; f.Xin = cl.Xin; f.xmod = cl.xmod; f.D_in = w.D_in; f.ls = d.lengthscales; f.var = d.variance;
-    f.kind = d.kernel_kind; f.Mp = w.Mp; f.D = w.D_out; f.N = N; f.Np = Np; f.Pp = Pp; f.S = (int)S; f.jitter = d.jitter;
-    f.var_out = (Fvars_host && Fvars_host[l]) ? Fvars_host[l] : nullptr; f.chol_in = cin;
+    f.V = w.fcfg >= 0 ? cl.A : tmp.t1; f.T = cl.T; f.Xin = cl.Xin; f.xmod = cl.xmod; f.D_in = w.D_in; f.ls = d.lengthscales;
+    f.var = d.variance; f.kind = d.kernel_kind; f.Mp = w.Mp; f.D = w.D_out; f.N = N; f.Np = Np; f.Pp = Pp; f.S = (int)S;
+    f.jitter = d.jitter; f.var_out = (Fvars_host && Fvars_host[l]) ? Fvars_host[l] : nullptr; f.chol_in = cin;
     const unsigned nt = (unsigned)(Np / kFcTile), nb = (unsigned)(S * w.D_out);
-    LAUNCH(fullcov_kernel, dim3(nt, nt, nb), 256, 0, f);
+    LAUNCH(fullcov_kernel, dim3(nt * (nt + 1) / 2, 1, nb), 256, 0, f);
     const bool last = l == nl - 1;
     const bool want_sample = !last || (Fs_host && Fs_host[l]);
     if (!want_sample) continue;
@@ -1847,7 +1853,16 @@ int dgp_propagate_full_cov(dgp_ctx* c, const dgp_model_desc* model, const double
                            double* const* Fmeans_host, double* const* Fvars_host) {
   if (!c || !model || !X) return DGP_ERR_ARG;
   CK(cudaSetDevice(c->device));
-  RC(planned(c, [&] { return run_full_cov(c, model, X, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host); }));
+  RC(planned(c, [&] { return run_full_cov(c, model, X, false, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host); }));
+  return check_chol(c);
+}
+
+int dgp_propagate_full_cov_snd(dgp_ctx* c, const dgp_model_desc* model, const double* X, int64_t N, int64_t S,
+                               const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
+                               double* const* Fmeans_host, double* const* Fvars_host) {
+  if (!c || !model || !X) return DGP_ERR_ARG;
+  CK(cudaSetDevice(c->device));
+  RC(planned(c, [&] { return run_full_cov(c, model, X, true, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host); }));
   return check_chol(c);
 }
 

@@ -23,13 +23,16 @@ struct FullCovArgs {
 
 constexpr int kFcTile = 32;
 
-// One 32 x 32 tile of a covariance block. The K term is the layer's stationary kernel on the input rows, or (EXT) the caller's
-// block Kff[s * kff_stride + i * N + j] (the supplied-matrix path: dgp_svgp_from_k_full_cov).
+// One 32 x 32 tile (rows i0.., columns j0..) of a covariance block. The K term is the layer's stationary kernel on the input rows,
+// or (EXT) the caller's block Kff[s * kff_stride + i * N + j] (the supplied-matrix path: dgp_svgp_from_k_full_cov).
+// mirror (i0 < j0): also store the transposed tile at (j0, i0). Without EXT every entry is symmetric bit for bit -- fma(a, b, c)
+// and fma(b, a, c) round the same exact product, the m order is the same, and x_i - x_j = -(x_j - x_i) exactly -- so the mirror is
+// what tile (j0, i0) would have computed.
 template <bool EXT>
-__device__ __forceinline__ void fullcov_tile(const FullCovArgs& a, const double* __restrict__ Kff, long kff_stride) {
+__device__ __forceinline__ void fullcov_tile(const FullCovArgs& a, const double* __restrict__ Kff, long kff_stride, int i0, int j0,
+                                             bool mirror) {
   __shared__ double vi[kFcTile][kFcTile + 1], vj[kFcTile][kFcTile + 1], ti[kFcTile][kFcTile + 1], tj[kFcTile][kFcTile + 1];
   const int s = blockIdx.z / a.D, d = blockIdx.z % a.D;
-  const int i0 = blockIdx.y * kFcTile, j0 = blockIdx.x * kFcTile;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // ty in 0..7: rows ty, ty + 8, ...
   const double* Td = a.T + (long)d * a.Mp * a.Pp;
   const long c0 = (long)s * a.N;
@@ -80,15 +83,34 @@ __device__ __forceinline__ void fullcov_tile(const FullCovArgs& a, const double*
       out_pad = cov + (i == j ? a.jitter : 0.0);
     }
     if (i < a.Np && j < a.Np) a.chol_in[((long)blockIdx.z * a.Np + i) * a.Np + j] = out_pad;
+    if (mirror) vi[ty + 8 * u][tx] = out_pad;   // off the diagonal tile i != j: out_pad is cov, or 0 on the padding
+  }
+  if (!mirror) return;
+  __syncthreads();
+  // transposed store, coalesced along the mirrored row: element (j0 + r, i0 + tx) = tile element (i0 + tx, j0 + r)
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int r = ty + 8 * u, i = j0 + r, j = i0 + tx;
+    const double v = vi[tx][r];
+    if (a.var_out && i < a.N && j < a.N) a.var_out[(((long)s * a.N + i) * a.N + j) * a.D + d] = v;
+    if (i < a.Np && j < a.Np) a.chol_in[((long)blockIdx.z * a.Np + i) * a.Np + j] = v;
   }
 }
 
-// grid: (Np / 32, Np / 32, S * D); block 32 x 8
-__global__ void __launch_bounds__(256) fullcov_kernel(FullCovArgs a) { fullcov_tile<false>(a, nullptr, 0); }
+// grid: (nt (nt + 1) / 2, 1, S * D) with nt = Np / 32; block 32 x 8. Block x is an upper-triangular tile (bi <= bj) in row-major
+// order; an off-diagonal tile also stores its mirror, so the Gram products run once per symmetric pair.
+__global__ void __launch_bounds__(256) fullcov_kernel(FullCovArgs a) {
+  const int nt = (int)(a.Np / kFcTile);
+  int t = blockIdx.x, bi = 0;
+  while (t >= nt - bi) { t -= nt - bi; ++bi; }
+  const int bj = bi + t;
+  fullcov_tile<false>(a, nullptr, 0, bi * kFcTile, bj * kFcTile, bi != bj);
+}
 
-// the same with the K term read from Kff [.][N][N]: kff_stride = N * N (one block per sample) or 0 (one block shared by all)
+// the same with the K term read from Kff [.][N][N]: kff_stride = N * N (one block per sample) or 0 (one block shared by all).
+// grid: (Np / 32, Np / 32, S * D), every tile computed: a caller's Kff need not be symmetric bit for bit.
 __global__ void __launch_bounds__(256) fullcov_ext_kernel(FullCovArgs a, const double* __restrict__ Kff, long kff_stride) {
-  fullcov_tile<true>(a, Kff, kff_stride);
+  fullcov_tile<true>(a, Kff, kff_stride, blockIdx.y * kFcTile, blockIdx.x * kFcTile, false);
 }
 
 // F[s][n][d] = mean[s][n][d] + sum_{n' <= n} L_{s,d}[n][n'] z[s][n'][d]        (utils/utils.py:50)

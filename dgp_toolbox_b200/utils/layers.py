@@ -35,8 +35,8 @@ class Layer(_Module):
         X = _lib.as_device(X, self.feature.Z.value.device)
         S, N, D = X.shape
         if full_cov:
-            mv = [self.conditional_ND(X[s].contiguous(), full_cov=True) for s in range(S)]
-            return [torch.stack([m for m, _ in mv]), torch.stack([v for _, v in mv])]
+            _, mean, var = self._propagate_full(X.contiguous(), S, None, 0, want_sample=False)
+            return [mean, var]
         mean, var = self.conditional_ND(X.reshape(S * N, D))
         return [m.reshape(S, N, self.num_outputs) for m in (mean, var)]
 
@@ -45,14 +45,17 @@ class Layer(_Module):
         X = _lib.as_device(X, self.feature.Z.value.device)
         S, N, _ = X.shape
         D = self.num_outputs
-        if full_cov:
-            # per sample: full N x N covariance per output and the Cholesky reparameterisation (utils/utils.py:43-52)
-            outs = []
-            for s in range(S):
-                zs = None if z is None else [_lib.as_device(z, X.device).reshape(S, N, D)[s:s + 1].contiguous()]
-                outs.append(self._propagate_full(X[s].contiguous(), 1, zs, int(seed) + s, layer_index))
-            return tuple(torch.cat([o[k] for o in outs]) for k in range(3))
         ctx = _lib.get_context(X.device)
+        if full_cov:
+            # per sample: full N x N covariance per output and the Cholesky reparameterisation (utils/utils.py:43-52), all S
+            # samples in one call. Without z, sample s draws the stream of seed + s (counter (n, 0, d, 0)), as one call per sample did.
+            if z is None:
+                z = torch.empty((S, N, D), dtype=torch.float64, device=X.device)
+                for s in range(S if N else 0):
+                    ctx.call("dgp_philox_normal", int(seed) + s, 0, 1, N, D, 0, _lib.ptr(z[s]))
+            else:
+                z = _lib.as_device(z, X.device).reshape(S, N, D).contiguous()
+            return self._propagate_full(X.contiguous(), S, [z], 0)
         if z is None:
             z = torch.empty((S, N, D), dtype=torch.float64, device=X.device)
             ctx.call("dgp_philox_normal", int(seed), int(layer_index), S, N, D, 0, _lib.ptr(z))
@@ -146,7 +149,7 @@ class SVGP_Layer(Layer):
         X = _lib.as_device(X, self.feature.Z.value.device)
         P = X.shape[0]
         if full_cov:
-            _, mean, var = self._propagate_full(X, 1, None, 0, 0, want_sample=False)
+            _, mean, var = self._propagate_full(X, 1, None, 0, want_sample=False)
             return mean[0], var[0]
         mean = torch.empty((P, self.num_outputs), dtype=torch.float64, device=X.device)
         var = torch.empty_like(mean)
@@ -156,9 +159,10 @@ class SVGP_Layer(Layer):
         _lib.get_context(X.device).call("dgp_conditional_nd", C.byref(d), _lib.ptr(X), P, _lib.ptr(mean), _lib.ptr(var))
         return mean, var
 
-    def _propagate_full(self, X, S, zs, seed, layer_index, want_sample=True):
-        """One-layer dgp_propagate_full_cov call: X [N, D_in] shared by the S samples -> (F, mean [S,N,D], var [S,N,N,D])."""
-        N, D = X.shape[0], self.num_outputs
+    def _propagate_full(self, X, S, zs, seed, want_sample=True):
+        """One-layer full_cov call: X [N, D_in] shared by the S samples (dgp_propagate_full_cov) or X [S, N, D_in] per sample
+        (dgp_propagate_full_cov_snd) -> (F, mean [S,N,D], var [S,N,N,D])."""
+        N, D = X.shape[-2], self.num_outputs
         mean = torch.empty((S, N, D), dtype=torch.float64, device=X.device)
         var = torch.empty((S, N, N, D), dtype=torch.float64, device=X.device)
         F = torch.empty((S, N, D), dtype=torch.float64, device=X.device) if want_sample else None
@@ -167,7 +171,8 @@ class SVGP_Layer(Layer):
         d, keep = self._desc()
         m = _lib.ModelDesc(1, C.pointer(d), None)
         zp = _lib.ptr_array(zs) if zs is not None else None
-        _lib.get_context(X.device).call("dgp_propagate_full_cov", C.byref(m), _lib.ptr(X), N, S, zp, int(seed), 0,
+        fn = "dgp_propagate_full_cov_snd" if X.dim() == 3 else "dgp_propagate_full_cov"
+        _lib.get_context(X.device).call(fn, C.byref(m), _lib.ptr(X), N, S, zp, int(seed), 0,
                                         _lib.ptr_array([F]), _lib.ptr_array([mean]), _lib.ptr_array([var]))
         return F, mean, var
 

@@ -329,10 +329,18 @@ int dgp_predict_moments(dgp_ctx* ctx, const dgp_model_desc* model, const double*
 /* DGP_Base.propagate(X, full_cov=True, S, zs) (models/dgp.py:34-63 with utils/layers.py:76-80,264-268,276 and utils/utils.py:43-52):
  * every layer's conditional is evaluated per sample with the full N x N covariance, samples are drawn with chol(var + jitter I) per
  * sample and output. Caller arrays (any may be NULL): Fs[l], Fmeans[l] [S, N, D_l]; Fvars[l] [S, N, N, D_l]. N <= 768 (one CTA
- * factorises an N x N block); layer shapes must be supported by the fused conditional kernel. zs / seed / n_offset as dgp_propagate. */
+ * factorises an N x N block). Layers the fused conditional kernel takes build the K(X_s, X_s) term inside the covariance tiles;
+ * other layers (dgp_set_fused(0), or a shape no fused configuration fits) run the unfused pipeline with the same covariance kernel,
+ * except white=True layers, which need the fused kernel. zs / seed / n_offset as dgp_propagate. */
 int dgp_propagate_full_cov(dgp_ctx* ctx, const dgp_model_desc* model, const double* X, int64_t N, int64_t S,
                            const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
                            double* const* Fmeans_host, double* const* Fvars_host);
+
+/* The same with the first layer's input given per sample: X [S, N, D_in] (Layer.conditional_SND / sample_from_conditional with
+ * full_cov=True on per-sample inputs: one call for all S samples). */
+int dgp_propagate_full_cov_snd(dgp_ctx* ctx, const dgp_model_desc* model, const double* X, int64_t N, int64_t S,
+                               const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
+                               double* const* Fmeans_host, double* const* Fvars_host);
 
 /* DGP_Base.E_log_p_Y (models/dgp.py:79-87): out [N, D_L] = mean over the S samples of the Gaussian variational expectations
  * (-0.5 log 2pi - 0.5 log s_n^2 - 0.5 ((Y - mu)^2 + var) / s_n^2, utils/utils.py:89-93) of the last layer's moments. */
