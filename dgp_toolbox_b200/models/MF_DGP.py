@@ -12,6 +12,7 @@ semantics (from the call sites utils/layers.py:208-213, MF_DGP.py:204-207,375-37
 from __future__ import annotations
 
 import ctypes as C
+import functools
 
 import numpy as np
 import torch
@@ -94,19 +95,20 @@ class MFLayer(_Module):
         return SVGPFromK.apply(ent["Ku"], Kuf, Kdiag, values.get(self.q_mu, self.q_mu.value), values.get(self.q_sqrt, self.q_sqrt.value),
                                ent["prep"])
 
-    def sample_from_conditional(self, X, z=None, values=None, draw=None, full_cov=False, shared_input=False):
+    def sample_from_conditional(self, X, z=None, values=None, draw=None, full_cov=False, shared_input=False, n_offset=0):
         """utils/layers.py:87-130: X [S, N, D] -> samples, mean [S, N, D_out], var [S, N, D_out] (full_cov=True: [S, N, N, D_out]).
-        shared_input: every sample's input is X[0] (the first application of a chain), so K(X_s, X_s) is one shared block."""
+        shared_input: every sample's input is X[0] (the first application of a chain), so K(X_s, X_s) is one shared block.
+        n_offset: global index of X's first point (a data-parallel shard), so the draws are those of the full batch (`draw_normal`)."""
         if full_cov:
-            return self._sample_full_cov(X, z, values, draw, shared_input)
+            return self._sample_full_cov(X, z, values, draw, shared_input, n_offset)
         S, N, D = X.shape
         mean, var, _ = self.conditional_ND(X.reshape(S * N, D), values)
         mean, var = mean.reshape(S, N, self.num_outputs), var.reshape(S, N, self.num_outputs)
         if z is None:
-            z = (draw or _default_draw(self.device))((S, N, self.num_outputs))
+            z = draw_normal(draw, self.device, (S, N, self.num_outputs), n_offset)
         return mean + z * torch.sqrt(var + DEFAULT_JITTER), mean, var
 
-    def _sample_full_cov(self, X, z, values, draw, shared_input):
+    def _sample_full_cov(self, X, z, values, draw, shared_input, n_offset=0):
         """conditional_SND(full_cov=True) + reparameterize(full_cov=True) (utils/layers.py:76-80,264-268,276; utils/utils.py:43-52):
         per sample the N x N covariance and a correlated draw, one dgp_svgp_from_k_full_cov call. Forward only. The draws are one
         `draw((S, N, D_out))`, as on the diagonal path, so seeds and recorded draws line up across the two modes."""
@@ -120,7 +122,7 @@ class MFLayer(_Module):
         Kuf = self.eval.K(Z, Xk.reshape(S * N, self.D).contiguous(), values)
         Kff = self.eval.K_blocks(Xk[:1] if shared_input else Xk, values)
         if z is None:
-            z = (draw or _default_draw(self.device))((S, N, self.num_outputs))
+            z = draw_normal(draw, self.device, (S, N, self.num_outputs), n_offset)
         z = z.expand(S, N, self.num_outputs)
         return svgp_from_k_full_cov(Ku, Kuf, Kff, values.get(self.q_mu, self.q_mu.value), values.get(self.q_sqrt, self.q_sqrt.value), z,
                                     DEFAULT_JITTER)
@@ -130,6 +132,12 @@ class MFLayer(_Module):
         values = values or {}
         Z = self.Zfull(values)
         return self.conditional_ND(Z[:1].detach(), values)[2]
+
+
+def _weighted_kl(layer, values, shard):
+    """A layer's KL term; in a data-parallel evaluation weighted so that the sum over the ranks is the term itself."""
+    kl = layer.KL(values)
+    return kl if shard is None else kl * shard.kl_weight
 
 
 def check_full_cov_inputs(X, values):
@@ -145,15 +153,16 @@ def _chol(K):
 
 
 class _PhiloxDraws:
-    """Default source of N(0, 1) draws: the library's Philox stream (dgp_philox_normal), one stream index per call."""
+    """Default source of N(0, 1) draws: the library's Philox stream (dgp_philox_normal), one stream index per call. The counter
+    carries the global point index n + n_offset, so draw((S, hi - lo, D), n_offset=lo) is draw((S, N, D))[:, lo:hi] bit for bit."""
 
     def __init__(self, device, seed=0):
         self.device, self.seed, self.calls = device, seed, 0
 
-    def __call__(self, shape):
+    def __call__(self, shape, n_offset=0):
         S, N, D = shape
         z = torch.empty(shape, dtype=torch.float64, device=self.device)
-        _lib.get_context(self.device).call("dgp_philox_normal", int(self.seed), int(self.calls), S, N, D, 0, _lib.ptr(z))
+        _lib.get_context(self.device).call("dgp_philox_normal", int(self.seed), int(self.calls), S, N, D, int(n_offset), _lib.ptr(z))
         self.calls += 1
         return z
 
@@ -165,6 +174,14 @@ def _default_draw(device):
     if device not in _draws:
         _draws[device] = _PhiloxDraws(device)
     return _draws[device]
+
+
+def draw_normal(draw, device, shape, n_offset=0):
+    """`draw(shape)` (default: the device's Philox draws) for points starting at global index n_offset. The keyword is passed only
+    when n_offset != 0, so a draw callable that takes just a shape (e.g. one replaying recorded draws) serves every unsharded run;
+    a data-parallel run (distributed.ShardedComposite) needs one that accepts `n_offset`, as the default Philox draw does."""
+    draw = draw or _default_draw(device)
+    return draw(shape, n_offset=n_offset) if n_offset else draw(shape)
 
 
 def sample(layer, Z, num_samples=50, values=None, draw=None):
@@ -217,9 +234,10 @@ class DGP_Base(_Module):
     def device(self):
         return self.layers[0].device
 
-    def propagate(self, X, full_cov=False, S=1, zs=None, values=None):
+    def propagate(self, X, full_cov=False, S=1, zs=None, values=None, n_offset=0):
         """MF_DGP.py:98-132: layer l >= 1 sees the input augmented with the previous layer's sample. full_cov=True: Fvars[l] is
-        [S, N, N, D_l] and the samples are correlated over the N points (forward only, N <= 768)."""
+        [S, N, N, D_l] and the samples are correlated over the N points (forward only, N <= 768). n_offset: global index of X's
+        first point (a data-parallel shard)."""
         if full_cov:
             check_full_cov_inputs(X, values)
         X = _lib.as_device(X, self.device)
@@ -230,13 +248,14 @@ class DGP_Base(_Module):
         for i, (layer, z) in enumerate(zip(self.layers, zs)):
             inp = F if i == 0 else torch.cat([sX, F], 2)
             z = None if z is None else _lib.as_device(z, self.device)
-            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=z, values=values, draw=self.draw, full_cov=full_cov, shared_input=i == 0)
+            F, Fmean, Fvar = layer.sample_from_conditional(inp, z=z, values=values, draw=self.draw, full_cov=full_cov, shared_input=i == 0,
+                                                           n_offset=n_offset)
             Fs.append(F); Fmeans.append(Fmean); Fvars.append(Fvar)
         return Fs, Fmeans, Fvars
 
-    def predict_f(self, X, full_cov=False, S=1, fidelity=None, values=None):
+    def predict_f(self, X, full_cov=False, S=1, fidelity=None, values=None, n_offset=0):
         """MF_DGP.py:134-149 (full_cov=True: the variance is [S, N, N, D])."""
-        _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values)
+        _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values, n_offset=n_offset)
         f = -1 if fidelity is None else fidelity
         return Fmeans[f], Fvars[f]
 
@@ -244,10 +263,10 @@ class DGP_Base(_Module):
         """MF_DGP.py:151-162."""
         return -0.5 * np.log(2 * np.pi) - 0.5 * torch.log(variance) - 0.5 * ((Y - Fmu) ** 2 + Fvar) / variance
 
-    def E_log_p_Y(self, X_f, Y_f, fidelity=None, values=None):
+    def E_log_p_Y(self, X_f, Y_f, fidelity=None, values=None, n_offset=0):
         """MF_DGP.py:164-197: the last fidelity uses the model's Gaussian likelihood, the others the White variance of their kernel."""
         values = values or {}
-        Fmean, Fvar = self.predict_f(X_f, S=self.num_samples, fidelity=fidelity, values=values)
+        Fmean, Fvar = self.predict_f(X_f, S=self.num_samples, fidelity=fidelity, values=values, n_offset=n_offset)
         Y = _lib.as_device(Y_f, self.device)[None]
         if fidelity == self.num_layers - 1:
             p = self.likelihood.likelihood.variance
@@ -264,8 +283,10 @@ class DGP_Base(_Module):
             f.Z_right = sample_Z_right(self.layers[0:i], zl, values, self.draw)
             f.Z = torch.cat([zl, f.Z_right], 1)
 
-    def ELBO(self, data, tf_sample_Z_right=True, values=None):
-        """MF_DGP.py:199-226 -> 0-d tensor (differentiable w.r.t. the leaves in `values`)."""
+    def ELBO(self, data, tf_sample_Z_right=True, values=None, shard=None):
+        """MF_DGP.py:199-226 -> 0-d tensor (differentiable w.r.t. the leaves in `values`). shard (distributed.CompositeShard): `data`
+        is one rank's part of the points; its data terms are partial sums and every KL term is weighted by shard.kl_weight, so the
+        sum over ranks is the full-batch ELBO. Z_right is re-sampled with the same draws on every rank."""
         if tf_sample_Z_right:
             self.refresh_Z_right(values)
         X, Y = data
@@ -274,19 +295,21 @@ class DGP_Base(_Module):
         for fidelity in range(self.num_layers):
             if self._train_upto_fidelity != -1 and fidelity > self._train_upto_fidelity:
                 continue
-            L = L + self.E_log_p_Y(X[fidelity], Y[fidelity], fidelity, values).sum()     # scale is identically 1 (:219-220)
-            KL = KL + self.layers[fidelity].KL(values)
+            off = 0 if shard is None else shard.offsets[fidelity]
+            L = L + self.E_log_p_Y(X[fidelity], Y[fidelity], fidelity, values, n_offset=off).sum()     # scale is identically 1 (:219-220)
+            KL = KL + _weighted_kl(self.layers[fidelity], values, shard)
         self.L, self.KL = L, KL
         return L - KL
 
     ELBO_closure = ELBO
 
-    def ELBO_and_grads(self, data, params=None):
-        """ELBO and its constrained-space gradients w.r.t. `params` (default: the trainable parameters): {Parameter: tensor}."""
+    def ELBO_and_grads(self, data, params=None, shard=None):
+        """ELBO and its constrained-space gradients w.r.t. `params` (default: the trainable parameters): {Parameter: tensor}.
+        shard: as in ELBO (this rank's un-reduced part)."""
         params = self.trainable_parameters if params is None else params
         values = {p: p.value.detach().clone().requires_grad_(True) for p in params}
         values[EVAL_CACHE] = {}
-        elbo = self.ELBO(data, values=values)
+        elbo = self.ELBO(data, values=values, shard=shard)
         grads = torch.autograd.grad(elbo, [values[p] for p in params], allow_unused=True)
         self._detach_features()
         return elbo.detach(), {p: (torch.zeros_like(p.value) if g is None else g) for p, g in zip(params, grads)}
@@ -359,12 +382,13 @@ class MultiFidelityDeepGP(_Module):
         with torch.no_grad():
             return self.model.ELBO((self._X, self._Y))
 
-    def _adam_phase(self, params, state, t0, iterations, lr, beta_1, beta_2, epsilon, messages):
+    def _adam_phase(self, params, state, t0, iterations, lr, beta_1, beta_2, epsilon, messages, evaluate=None):
         """One phase of the reference's loops (:381-388): ELBO + gradients through the library calls, then the library's fused Adam
         launch (dgp_adam_step with the GPflow bijectors) on a flat gradient buffer."""
         m = self.model
+        evaluate = evaluate or functools.partial(m.ELBO_and_grads, (self._X, self._Y))
         for it in range(iterations):
-            elbo, grads = m.ELBO_and_grads((self._X, self._Y), params)
+            elbo, grads = evaluate(params)
             flat = torch.cat([grads[p].reshape(-1) for p in params]) if params else torch.zeros(1, dtype=torch.float64, device=m.device)
             if params:
                 _adam_step(m.device, params, flat, state, t0 + it, lr, beta_1, beta_2, epsilon)
@@ -373,8 +397,10 @@ class MultiFidelityDeepGP(_Module):
         return t0 + iterations
 
     def optimize_adam(self, lr=0.01, iterations1=2000, iterations2=5000, iterations3=7500, beta_1=0.9, beta_2=0.999, epsilon=1e-07,
-                      messages=500):
-        """MF_DGP.py:345-424: three phases (kernel parameters; + inducing inputs; + variational parameters and likelihood variance)."""
+                      messages=500, evaluate=None):
+        """MF_DGP.py:345-424: three phases (kernel parameters; + inducing inputs; + variational parameters and likelihood variance).
+        evaluate: callable `params -> (elbo, grads)` used instead of `model.ELBO_and_grads` on this object's data (the data-parallel
+        evaluation of distributed.ShardedComposite)."""
         m = self.model
         for i, layer in enumerate(m.layers[:-1]):
             layer.q_mu.assign(self._Y[i]); set_trainable(layer.q_mu, False)
@@ -389,25 +415,26 @@ class MultiFidelityDeepGP(_Module):
             set_trainable(layer.feature.Z_left, False)
         state = {}        # per-parameter (m, v) of tf.optimizers.Adam: ONE optimiser serves the three phases (:360)
         print('Training part 1')
-        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr, beta_1, beta_2, epsilon, messages)
+        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
         print('Training part 2')
-        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr, beta_1, beta_2, epsilon, messages)
+        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.likelihood.likelihood.variance, True)
         for layer in m.layers:
             set_trainable(layer.q_mu, True); set_trainable(layer.q_sqrt, True)
         print('Training part 3')
-        self._adam_phase(m.trainable_parameters, state, t, iterations3, lr, beta_1, beta_2, epsilon, messages)
+        self._adam_phase(m.trainable_parameters, state, t, iterations3, lr, beta_1, beta_2, epsilon, messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
 
 
     def optimize_nat_adam(self, lr_adam=0.01, lr_gamma=0.01, iterations1=2000, iterations2=5000, iterations3=7500, beta_1=0.9, beta_2=0.999,
-                          epsilon=1e-07, messages=500):
+                          epsilon=1e-07, messages=500, evaluate=None):
         """MF_DGP.py:426-512: Adam on the kernel parameters; + inducing inputs; then per iteration an Adam step on those and the
-        likelihood variance plus a natural-gradient step on every layer's (q_mu, q_sqrt) (two ELBO evaluations per iteration)."""
+        likelihood variance plus a natural-gradient step on every layer's (q_mu, q_sqrt) (two ELBO evaluations per iteration).
+        evaluate: as in optimize_adam."""
         m = self.model
         data = (self._X, self._Y)
         for i, layer in enumerate(m.layers[:-1]):
@@ -422,27 +449,28 @@ class MultiFidelityDeepGP(_Module):
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, False)
         state = {}
-        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr_adam, beta_1, beta_2, epsilon, messages)
+        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr_adam, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
-        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr_adam, beta_1, beta_2, epsilon, messages)
+        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr_adam, beta_1, beta_2, epsilon, messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         set_trainable(m.likelihood.likelihood.variance, True)
-        nat_adam_phase(m, data, state, t, iterations3, lr_adam, beta_1, beta_2, epsilon, lr_gamma, list(m.layers), messages)
+        nat_adam_phase(m, data, state, t, iterations3, lr_adam, beta_1, beta_2, epsilon, lr_gamma, list(m.layers), messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         _lib.get_context(m.device).check()
 
 
-def natgrad_pairs(model, data, gamma, layers):
+def natgrad_pairs(model, data, gamma, layers, evaluate=None):
     """GPflow `NaturalGradient(gamma).minimize(lambda: -ELBO(data), var_list=[(q_mu, q_sqrt) of layers])` (MF_DGP.py:501-507,
     MF_DGP_EM.py, MO_DGP.py:480-487): a FRESH ELBO evaluation (new draws, Z_right re-sampled) differentiated w.r.t. the variational
     parameters through the library's layer adjoints, then one dgp_natgrad_pairs call (XiNat step, batched over layers and outputs,
-    in place). Returns that evaluation's ELBO."""
+    in place). Returns that evaluation's ELBO. evaluate: callable `params -> (elbo, grads)` in place of
+    `model.ELBO_and_grads(data, params)`."""
     params = [p for l in layers for p in (l.q_mu, l.q_sqrt)]
-    elbo, grads = model.ELBO_and_grads(data, params)
+    elbo, grads = (evaluate or functools.partial(model.ELBO_and_grads, data))(params)
     arr = (_lib.NatPair * len(layers))()
     keep = []
     for i, l in enumerate(layers):
@@ -455,15 +483,17 @@ def natgrad_pairs(model, data, gamma, layers):
     return elbo
 
 
-def nat_adam_phase(model, data, state, t0, iterations, lr, beta_1, beta_2, epsilon, gamma, layers, messages):
+def nat_adam_phase(model, data, state, t0, iterations, lr, beta_1, beta_2, epsilon, gamma, layers, messages, evaluate=None):
     """Part 3 of the reference's optimize_nat_adam loops (MF_DGP.py:499-509): per iteration one Adam step on the trainable
-    (non-variational) parameters and one natural-gradient step on `layers`, each with its own ELBO evaluation."""
+    (non-variational) parameters and one natural-gradient step on `layers`, each with its own ELBO evaluation (both through
+    `evaluate`, as in natgrad_pairs)."""
+    evaluate = evaluate or functools.partial(model.ELBO_and_grads, data)
     for it in range(iterations):
         params = model.trainable_parameters
-        elbo, grads = model.ELBO_and_grads(data, params)
+        elbo, grads = evaluate(params)
         if params:
             _adam_step(model.device, params, torch.cat([grads[p].reshape(-1) for p in params]), state, t0 + it, lr, beta_1, beta_2, epsilon)
-        natgrad_pairs(model, data, gamma, layers)
+        natgrad_pairs(model, data, gamma, layers, evaluate)
         if it % messages == 0:
             print(f"ELBO: {float(elbo)}")
     return t0 + iterations

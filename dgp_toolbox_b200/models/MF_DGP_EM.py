@@ -5,13 +5,15 @@ second Gaussian likelihood), the fidelity layers see `[H_k, f_{l-1}]` with `H_k`
 Same machinery as models/MF_DGP.py: kernels, layer conditionals / KL and all adjoints are library calls chained by torch.autograd."""
 from __future__ import annotations
 
+import functools
+
 import numpy as np
 import torch
 
 from .. import _lib
 from ..composite import EVAL_CACHE, RBF, LinearKernel, White
 from ..gpflow_shim import Gaussian, _Module, set_trainable
-from .MF_DGP import MFLayer, _Lik, _adam_step, check_full_cov_inputs, sample
+from .MF_DGP import MFLayer, _Lik, _adam_step, _weighted_kl, check_full_cov_inputs, sample
 
 
 def sample_Z_right(layers, layers_red, Z, values=None, draw=None, num_samples=50):
@@ -28,6 +30,11 @@ def sample_Z_right(layers, layers_red, Z, values=None, draw=None, num_samples=50
         else:
             Z_right = sample(layer, torch.cat([Hs[-(i + 1)], Z_right], 1), num_samples, values, draw)
     return Z_right
+
+
+def projection_scale(counts, fidelity):
+    """Weight n(X[l+1]) / n(X[l]) of fidelity l's projection term (MF_DGP_EM.py:283), from the point counts of the whole batch."""
+    return float(counts[fidelity + 1]) / float(counts[fidelity])
 
 
 def init_layers_mf(X, Z, W, kernels, kernels_red, num_outputs=None, draw=None):
@@ -61,10 +68,10 @@ class DGP_Base(_Module):
     def device(self):
         return self.layers[0].device
 
-    def propagate(self, X, full_cov=False, S=1, zs=None, ws=None, fidelity_dim=None, project=False, values=None):
+    def propagate(self, X, full_cov=False, S=1, zs=None, ws=None, fidelity_dim=None, project=False, values=None, n_offset=0):
         """MF_DGP_EM.py:120-168: X lives in the input space of fidelity `fidelity_dim` (default: the highest). full_cov=True: the
         variances (Hvars with project=True) are [S, N, N, D] and the samples are correlated over the N points (forward only,
-        N <= 768)."""
+        N <= 768). n_offset: global index of X's first point (a data-parallel shard)."""
         if full_cov:
             check_full_cov_inputs(X, values)
         X = _lib.as_device(X, self.device)
@@ -78,7 +85,7 @@ class DGP_Base(_Module):
         # the first application of the chain sees X itself for every sample: the first projection layer, or layer 0 without one
         for j, (layer_red, w) in enumerate(zip(self.layers_red[L - fidelity_dim:], ws[L - fidelity_dim:])):
             H, Hmean, Hvar = layer_red.sample_from_conditional(H, z=dev(w), values=values, draw=self.draw, full_cov=full_cov,
-                                                               shared_input=j == 0)
+                                                               shared_input=j == 0, n_offset=n_offset)
             Hs.append(H); Hmeans.append(Hmean); Hvars.append(Hvar)
         if project:
             return Hs, Hmeans, Hvars
@@ -86,19 +93,19 @@ class DGP_Base(_Module):
         for i, (layer, z) in enumerate(zip(self.layers[:fidelity_dim + 1], zs[:fidelity_dim + 1])):
             inp = Hs[-1] if i == 0 else torch.cat([Hs[-(i + 1)], F], 2)
             F, Fmean, Fvar = layer.sample_from_conditional(inp, z=dev(z), values=values, draw=self.draw, full_cov=full_cov,
-                                                           shared_input=i == 0 and len(Hs) == 1)
+                                                           shared_input=i == 0 and len(Hs) == 1, n_offset=n_offset)
             Fs.append(F); Fmeans.append(Fmean); Fvars.append(Fvar)
         return Fs, Fmeans, Fvars
 
-    def predict_f(self, X, full_cov=False, S=1, fidelity=None, fidelity_dim=None, values=None):
+    def predict_f(self, X, full_cov=False, S=1, fidelity=None, fidelity_dim=None, values=None, n_offset=0):
         """`full_cov` is accepted and not passed on (so is `project`'s): both return the diagonal moments whatever it is. Whether the
         reference passes it on is not pinned by a test of the reference's own code; propagate(full_cov=True) gives the covariances."""
-        _, Fmeans, Fvars = self.propagate(X, S=S, fidelity_dim=fidelity_dim, values=values)
+        _, Fmeans, Fvars = self.propagate(X, S=S, fidelity_dim=fidelity_dim, values=values, n_offset=n_offset)
         f = -1 if fidelity is None else fidelity
         return Fmeans[f], Fvars[f]
 
-    def project(self, X, full_cov=False, S=1, fidelity=None, fidelity_dim=None, values=None):
-        _, Hmeans, Hvars = self.propagate(X, S=S, fidelity_dim=fidelity_dim, project=True, values=values)
+    def project(self, X, full_cov=False, S=1, fidelity=None, fidelity_dim=None, values=None, n_offset=0):
+        _, Hmeans, Hvars = self.propagate(X, S=S, fidelity_dim=fidelity_dim, project=True, values=values, n_offset=n_offset)
         f = -1 if fidelity is None else fidelity
         return Hmeans[f], Hvars[f]
 
@@ -106,15 +113,17 @@ class DGP_Base(_Module):
     def _gauss(Fmu, Fvar, Y, variance):
         return -0.5 * np.log(2 * np.pi) - 0.5 * torch.log(variance) - 0.5 * ((Y - Fmu) ** 2 + Fvar) / variance
 
-    def E_log_p_Y(self, X_f, Y_f, fidelity=None, fidelity_dim=None, project=False, values=None):
+    def E_log_p_Y(self, X_f, Y_f, fidelity=None, fidelity_dim=None, project=False, values=None, n_offset=0):
         """MF_DGP_EM.py:217-255."""
         values = values or {}
         Y = _lib.as_device(Y_f, self.device)[None]
         if project:
-            Hmean, Hvar = self.project(X_f, S=self.num_samples, fidelity=fidelity, fidelity_dim=fidelity_dim, values=values)
+            Hmean, Hvar = self.project(X_f, S=self.num_samples, fidelity=fidelity, fidelity_dim=fidelity_dim, values=values,
+                                       n_offset=n_offset)
             p = self.likelihood_projection.likelihood.variance
             return self._gauss(Hmean, Hvar, Y, values.get(p, p.value)).mean(0)
-        Fmean, Fvar = self.predict_f(X_f, S=self.num_samples, fidelity=fidelity, fidelity_dim=fidelity_dim, values=values)
+        Fmean, Fvar = self.predict_f(X_f, S=self.num_samples, fidelity=fidelity, fidelity_dim=fidelity_dim, values=values,
+                                     n_offset=n_offset)
         p = self.likelihood.likelihood.variance if fidelity == self.num_layers - 1 else self.layers[fidelity].kern.kernels[-1].variance
         return self._gauss(Fmean, Fvar, Y, values.get(p, p.value)).mean(0)
 
@@ -127,31 +136,35 @@ class DGP_Base(_Module):
             f.Z_right = sample_Z_right(self.layers[0:i], self.layers_red[L - i:], zl, values, self.draw)
             f.Z = torch.cat([zl, f.Z_right], 1)
 
-    def ELBO(self, data, values=None):
-        """MF_DGP_EM.py:257-297, as written: the projection term of fidelity l is scaled by n(X[l+1]) / n(X[l])."""
+    def ELBO(self, data, values=None, shard=None):
+        """MF_DGP_EM.py:257-297, as written: the projection term of fidelity l is scaled by n(X[l+1]) / n(X[l]). shard
+        (distributed.CompositeShard): `data` is one rank's part of the points (X_red[l] split as X[l+1]); data terms are partial
+        sums, the projection scale uses the global point counts and every KL term is weighted by shard.kl_weight."""
         X, Y, X_red = data
         self.refresh_Z_right(values)
         Lf = KL = L_red = KL_red = 0.0
+        counts = [np.shape(x)[0] for x in X] if shard is None else shard.counts
+        off = [0] * len(X) if shard is None else shard.offsets
         for fidelity in range(self.num_layers):
             if self._train_upto_fidelity != -1 and fidelity > self._train_upto_fidelity:
                 continue
-            Lf = Lf + self.E_log_p_Y(X[fidelity], Y[fidelity], fidelity, fidelity_dim=fidelity, values=values).sum()
-            KL = KL + self.layers[fidelity].KL(values)
+            Lf = Lf + self.E_log_p_Y(X[fidelity], Y[fidelity], fidelity, fidelity_dim=fidelity, values=values, n_offset=off[fidelity]).sum()
+            KL = KL + _weighted_kl(self.layers[fidelity], values, shard)
             if fidelity < self.num_layers - 1:
-                scale = float(np.shape(X[fidelity + 1])[0]) / float(np.shape(X[fidelity])[0])
+                scale = projection_scale(counts, fidelity)
                 L_red = L_red + self.E_log_p_Y(X[fidelity + 1], X_red[fidelity], fidelity, fidelity_dim=fidelity + 1, project=True,
-                                               values=values).sum() * scale
-                KL_red = KL_red + self.layers_red[fidelity].KL(values)
+                                               values=values, n_offset=off[fidelity + 1]).sum() * scale
+                KL_red = KL_red + _weighted_kl(self.layers_red[fidelity], values, shard)
         self.L, self.KL, self.L_red, self.KL_red = Lf, KL, L_red, KL_red
         return Lf + L_red - KL - KL_red
 
     ELBO_closure = ELBO
 
-    def ELBO_and_grads(self, data, params=None):
+    def ELBO_and_grads(self, data, params=None, shard=None):
         params = self.trainable_parameters if params is None else params
         values = {p: p.value.detach().clone().requires_grad_(True) for p in params}
         values[EVAL_CACHE] = {}
-        elbo = self.ELBO(data, values=values)
+        elbo = self.ELBO(data, values=values, shard=shard)
         grads = torch.autograd.grad(elbo, [values[p] for p in params], allow_unused=True)
         for layer in self.layers[1:]:
             layer.feature.Z_right = layer.feature.Z_right.detach()
@@ -205,11 +218,12 @@ class MultiFidelityDeepGP_EM(_Module):
         with torch.no_grad():
             return self.model.ELBO((self._X, self._Y, self._X_red))
 
-    def _phase(self, state, t0, iterations, lr, beta_1, beta_2, epsilon, messages):
+    def _phase(self, state, t0, iterations, lr, beta_1, beta_2, epsilon, messages, evaluate=None):
         m = self.model
         params = m.trainable_parameters
+        evaluate = evaluate or functools.partial(m.ELBO_and_grads, (self._X, self._Y, self._X_red))
         for it in range(iterations):
-            elbo, grads = m.ELBO_and_grads((self._X, self._Y, self._X_red), params)
+            elbo, grads = evaluate(params)
             if params:
                 _adam_step(m.device, params, torch.cat([grads[p].reshape(-1) for p in params]), state, t0 + it, lr, beta_1, beta_2, epsilon)
             if it % messages == 0:
@@ -217,8 +231,9 @@ class MultiFidelityDeepGP_EM(_Module):
         return t0 + iterations
 
     def optimize_adam(self, lr=0.01, iterations1=2000, iterations2=5000, iterations3=7500, beta_1=0.9, beta_2=0.999, epsilon=1e-07,
-                      messages=500):
-        """MF_DGP_EM.py:417-480."""
+                      messages=500, evaluate=None):
+        """MF_DGP_EM.py:417-480. evaluate: callable `params -> (elbo, grads)` used instead of `model.ELBO_and_grads` on this object's
+        data (the data-parallel evaluation of distributed.ShardedComposite)."""
         m = self.model
         for i, layer in enumerate(m.layers[:-1]):
             layer.q_mu.assign(self._Y[i]); set_trainable(layer.q_mu, False)
@@ -235,22 +250,22 @@ class MultiFidelityDeepGP_EM(_Module):
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, False)
         state = {}
-        t = self._phase(state, 1, iterations1, lr, beta_1, beta_2, epsilon, messages)
+        t = self._phase(state, 1, iterations1, lr, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
-        t = self._phase(state, t, iterations2, lr, beta_1, beta_2, epsilon, messages)
+        t = self._phase(state, t, iterations2, lr, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.likelihood.likelihood.variance, True)
         for layer in m.layers:
             set_trainable(layer.q_mu, True); set_trainable(layer.q_sqrt, True)
-        self._phase(state, t, iterations3, lr, beta_1, beta_2, epsilon, messages)
+        self._phase(state, t, iterations3, lr, beta_1, beta_2, epsilon, messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
 
     def optimize_nat_adam(self, lr_adam=0.01, lr_gamma=0.01, iterations1=2000, iterations2=5000, iterations3=7500, beta_1=0.9, beta_2=0.999,
-                          epsilon=1e-07, messages=500):
+                          epsilon=1e-07, messages=500, evaluate=None):
         """MF_DGP_EM.py:501-582, as written: start scalings 1e-3 / 1e-5, the likelihood variances stay frozen in part 3 (:563), the
-        natural-gradient step covers the fidelity layers and the projection layers (:564-565)."""
+        natural-gradient step covers the fidelity layers and the projection layers (:564-565). evaluate: as in optimize_adam."""
         from .MF_DGP import nat_adam_phase
         m = self.model
         data = (self._X, self._Y, self._X_red)
@@ -271,14 +286,15 @@ class MultiFidelityDeepGP_EM(_Module):
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, False)
         state = {}
-        t = self._phase(state, 1, iterations1, lr_adam, beta_1, beta_2, epsilon, messages)
+        t = self._phase(state, 1, iterations1, lr_adam, beta_1, beta_2, epsilon, messages, evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
-        t = self._phase(state, t, iterations2, lr_adam, beta_1, beta_2, epsilon, messages)
+        t = self._phase(state, t, iterations2, lr_adam, beta_1, beta_2, epsilon, messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
-        nat_adam_phase(m, data, state, t, iterations3, lr_adam, beta_1, beta_2, epsilon, lr_gamma, list(m.layers) + list(m.layers_red), messages)
+        nat_adam_phase(m, data, state, t, iterations3, lr_adam, beta_1, beta_2, epsilon, lr_gamma, list(m.layers) + list(m.layers_red), messages,
+                       evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         _lib.get_context(m.device).check()

@@ -18,6 +18,8 @@ DEVIATION below and unpinned:
 """
 from __future__ import annotations
 
+import functools
+
 import numpy as np
 import torch
 
@@ -25,12 +27,12 @@ from .. import _lib
 from ..composite import RBF, LinearKernel, White
 from ..gpflow_shim import Gaussian, _Module, set_trainable
 from . import MF_DGP as _MF
-from .MF_DGP import MFLayer, _adam_step, _default_draw, sample
+from .MF_DGP import MFLayer, _adam_step, _weighted_kl, draw_normal, sample
 
 
-def _start_column(n, device, draw):
-    """tf.random.normal([n, 1]) of MO_DGP.py:104: one draw per call, shared by all S samples."""
-    return (draw or _default_draw(device))((1, n, 1)).reshape(n, 1)
+def _start_column(n, device, draw, n_offset=0):
+    """tf.random.normal([n, 1]) of MO_DGP.py:104: one draw per call, shared by all S samples (n_offset: as in draw_normal)."""
+    return draw_normal(draw, device, (1, n, 1), n_offset).reshape(n, 1)
 
 
 def sample_Z_right(layers, Z, values=None, draw=None, num_samples=50):
@@ -67,12 +69,13 @@ class DGP_Base(_MF.DGP_Base):
         self._train_upto_objective = -1
         self.loop = loop
 
-    def propagate(self, X, full_cov=False, S=1, zs=None, values=None):
+    def propagate(self, X, full_cov=False, S=1, zs=None, values=None, n_offset=0):
         """MO_DGP.py:88-122 -> (Fs, Fmeans, Fvars), two entries each (objective 0, objective 1), [S, N, 1]. The chain starts from one
         N(0,1) column per point (shared by the S samples), runs layer 0, then alternates layers 1, 0, 1, 0 ... (2 loop applications;
         loop = 0: layer 1 once), reads objective 0 from the last application and objective 1 from one more application of layer 1.
         `zs[k]`, when given, is reused by every application of layer k, as in the reference. full_cov=True: Fvars are [S, N, N, 1]
-        and the samples are correlated over the N points (forward only, N <= 768)."""
+        and the samples are correlated over the N points (forward only, N <= 768). n_offset: global index of X's first point (a
+        data-parallel shard)."""
         if full_cov:
             _MF.check_full_cov_inputs(X, values)
         if not (isinstance(X, torch.Tensor) and X.requires_grad):      # a leaf the caller differentiates w.r.t. (EHVI_with_grad)
@@ -82,9 +85,9 @@ class DGP_Base(_MF.DGP_Base):
 
         def apply(k, F, shared=False):
             return self.layers[k].sample_from_conditional(torch.cat([sX, F], 2), z=zs[k], values=values, draw=self.draw,
-                                                          full_cov=full_cov, shared_input=shared)
+                                                          full_cov=full_cov, shared_input=shared, n_offset=n_offset)
 
-        F = _start_column(X.shape[0], self.device, self.draw)[None].expand(S, -1, -1)
+        F = _start_column(X.shape[0], self.device, self.draw, n_offset)[None].expand(S, -1, -1)
         F, Fmean, Fvar = apply(0, F, shared=True)      # [x, start column] is the same for every sample
         if self.loop == 0:
             F, Fmean, Fvar = apply(1, F)
@@ -96,19 +99,19 @@ class DGP_Base(_MF.DGP_Base):
         Fs.append(F); Fmeans.append(Fmean); Fvars.append(Fvar)
         return Fs, Fmeans, Fvars
 
-    def predict_f(self, X, full_cov=False, S=1, objective=None, values=None, fidelity=None):
+    def predict_f(self, X, full_cov=False, S=1, objective=None, values=None, fidelity=None, n_offset=0):
         """MO_DGP.py:124-138 (full_cov=True: the variance is [S, N, N, 1])."""
         objective = fidelity if objective is None else objective
-        _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values)
+        _, Fmeans, Fvars = self.propagate(X, full_cov=full_cov, S=S, values=values, n_offset=n_offset)
         o = -1 if objective is None else objective
         return Fmeans[o], Fvars[o]
 
     _likelihood_at_objective = _MF.DGP_Base._likelihood_at_fidelity      # MO_DGP.py:140-151
 
-    def E_log_p_Y(self, X_o, Y_o, objective=None, values=None):
+    def E_log_p_Y(self, X_o, Y_o, objective=None, values=None, n_offset=0):
         """MO_DGP.py:153-185: objective 1 (the last layer) uses the model's Gaussian likelihood, objective 0 the White variance of
         its kernel."""
-        return super().E_log_p_Y(X_o, Y_o, objective, values)
+        return super().E_log_p_Y(X_o, Y_o, objective, values, n_offset)
 
     def refresh_Z_right(self, values=None):
         """MO_DGP.py:192-195 (with the DEVIATION of sample_Z_right)."""
@@ -121,27 +124,29 @@ class DGP_Base(_MF.DGP_Base):
             f.Z_right = sample_Z_right(self.layers[0:i], zl, values, self.draw)
             f.Z = torch.cat([zl, f.Z_right], 1)
 
-    def ELBO(self, data, tf_sample_Z_right=True, values=None):
-        """MO_DGP.py:187-216: every objective's term runs its own chain (`predict_f(objective)`); scale is identically 1 (:207-208)."""
+    def ELBO(self, data, tf_sample_Z_right=True, values=None, shard=None):
+        """MO_DGP.py:187-216: every objective's term runs its own chain (`predict_f(objective)`); scale is identically 1 (:207-208).
+        shard: as in MF_DGP.DGP_Base.ELBO (one rank's part of every objective's points)."""
         if tf_sample_Z_right:
             self.refresh_Z_right(values)
         X, Y = data
         L = 0.0
         KL = 0.0
         for objective in range(self.num_layers):
-            L = L + self.E_log_p_Y(X[objective], Y[objective], objective, values).sum()
-            KL = KL + self.layers[objective].KL(values)
+            off = 0 if shard is None else shard.offsets[objective]
+            L = L + self.E_log_p_Y(X[objective], Y[objective], objective, values, n_offset=off).sum()
+            KL = KL + _weighted_kl(self.layers[objective], values, shard)
         self.L, self.KL = L, KL
         return L - KL
 
     ELBO_closure = ELBO
 
-    def ELBO_and_grads(self, data, params=None, tf_sample_Z_right=True):
+    def ELBO_and_grads(self, data, params=None, tf_sample_Z_right=True, shard=None):
         """ELBO and its constrained-space gradients w.r.t. `params` (default: the trainable parameters): {Parameter: tensor}."""
         params = self.trainable_parameters if params is None else params
         values = {p: p.value.detach().clone().requires_grad_(True) for p in params}
         values[_MF.EVAL_CACHE] = {}
-        elbo = self.ELBO(data, tf_sample_Z_right=tf_sample_Z_right, values=values)
+        elbo = self.ELBO(data, tf_sample_Z_right=tf_sample_Z_right, values=values, shard=shard)
         grads = torch.autograd.grad(elbo, [values[p] for p in params], allow_unused=True)
         self._detach_features()
         return elbo.detach(), {p: (torch.zeros_like(p.value) if g is None else g) for p, g in zip(params, grads)}
@@ -221,10 +226,11 @@ class MultiObjDeepGP(_Module):
         with torch.no_grad():
             return self.model.ELBO((self._X, self._Y))
 
-    def _adam_phase(self, params, state, t0, iterations, lr, epsilon, messages, tf_sample_Z_right=True):
+    def _adam_phase(self, params, state, t0, iterations, lr, epsilon, messages, tf_sample_Z_right=True, evaluate=None):
         m = self.model
+        evaluate = evaluate or functools.partial(m.ELBO_and_grads, (self._X, self._Y))
         for it in range(iterations):
-            elbo, grads = m.ELBO_and_grads((self._X, self._Y), params, tf_sample_Z_right=tf_sample_Z_right)
+            elbo, grads = evaluate(params, tf_sample_Z_right=tf_sample_Z_right)
             if params:
                 flat = torch.cat([grads[p].reshape(-1) for p in params])
                 _adam_step(m.device, params, flat, state, t0 + it, lr, 0.9, 0.999, epsilon)
@@ -232,10 +238,12 @@ class MultiObjDeepGP(_Module):
                 print(f"ELBO: {float(elbo)}")
         return t0 + iterations
 
-    def optimize_adam(self, lr=0.01, iterations1=2000, iterations2=5000, iterations3=7500, messages=500):
+    def optimize_adam(self, lr=0.01, iterations1=2000, iterations2=5000, iterations3=7500, messages=500, evaluate=None):
         """MO_DGP.py:344-417, as written: tf.optimizers.Adam(lr, epsilon=1e-8) shared by three phases (kernel parameters -- and, as
         written, layer 0's q_sqrt, which the reference never freezes; + inducing inputs; + variational parameters and the likelihood
-        variance), Z_right re-sampled at every ELBO evaluation and once more after each phase."""
+        variance), Z_right re-sampled at every ELBO evaluation and once more after each phase. evaluate: callable
+        `params, tf_sample_Z_right=True -> (elbo, grads)` used instead of `model.ELBO_and_grads` on this object's data (the
+        data-parallel evaluation of distributed.ShardedComposite)."""
         m = self.model
         m.layers[0].q_mu.assign(self._Y[0]); set_trainable(m.layers[0].q_mu, False)
         for i, layer in enumerate(m.layers[1:]):
@@ -249,28 +257,29 @@ class MultiObjDeepGP(_Module):
             set_trainable(layer.feature.Z_left, False)
         state = {}
         print('Training part 1')
-        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr, 1e-8, messages)
+        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr, 1e-8, messages, evaluate=evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
         with torch.no_grad():
             m.refresh_Z_right()
         print('Training part 2')
-        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr, 1e-8, messages)
+        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr, 1e-8, messages, evaluate=evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         set_trainable(m.likelihood.likelihood.variance, True)
         for layer in m.layers:
             set_trainable(layer.q_mu, True); set_trainable(layer.q_sqrt, True)
         print('Training part 3')
-        self._adam_phase(m.trainable_parameters, state, t, iterations3, lr, 1e-8, messages)
+        self._adam_phase(m.trainable_parameters, state, t, iterations3, lr, 1e-8, messages, evaluate=evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         _lib.get_context(m.device).check()
 
-    def optimize_nat_adam(self, lr_adam=0.01, lr_gamma=0.01, iterations1=2000, iterations2=5000, iterations3=7500, messages=500):
+    def optimize_nat_adam(self, lr_adam=0.01, lr_gamma=0.01, iterations1=2000, iterations2=5000, iterations3=7500, messages=500,
+                          evaluate=None):
         """MO_DGP.py:418-494, as written: part 1 without re-sampling Z_right (:462), start scalings 1e-2, then Adam + a natural-gradient
-        step on both layers per iteration."""
+        step on both layers per iteration. evaluate: as in optimize_adam."""
         from .MF_DGP import nat_adam_phase
         m = self.model
         m.layers[0].q_mu.assign(self._Y[0]); set_trainable(m.layers[0].q_mu, False)
@@ -285,17 +294,18 @@ class MultiObjDeepGP(_Module):
             set_trainable(layer.feature.Z_left, False)
         state = {}
         print('Training part 1')
-        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr_adam, 1e-8, messages, tf_sample_Z_right=False)
+        t = self._adam_phase(m.trainable_parameters, state, 1, iterations1, lr_adam, 1e-8, messages, tf_sample_Z_right=False,
+                             evaluate=evaluate)
         set_trainable(m.layers[0].feature.Z, True)
         for layer in m.layers[1:]:
             set_trainable(layer.feature.Z_left, True)
         print('Training part 2')
-        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr_adam, 1e-8, messages)
+        t = self._adam_phase(m.trainable_parameters, state, t, iterations2, lr_adam, 1e-8, messages, evaluate=evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         set_trainable(m.likelihood.likelihood.variance, True)
         print('Training part 3')
-        nat_adam_phase(m, (self._X, self._Y), state, t, iterations3, lr_adam, 0.9, 0.999, 1e-8, lr_gamma, list(m.layers), messages)
+        nat_adam_phase(m, (self._X, self._Y), state, t, iterations3, lr_adam, 0.9, 0.999, 1e-8, lr_gamma, list(m.layers), messages, evaluate)
         with torch.no_grad():
             m.refresh_Z_right()
         _lib.get_context(m.device).check()
