@@ -122,6 +122,66 @@ class EI(Infill_criteria):
         return self.x_opt
 
 
+class qEI(Infill_criteria):
+    """Batch expected improvement of q points: EI.run(analytic=False)'s mean_s max(y_min - F, 0) (Infill_criteria.py:49-51) with
+    F replaced by the minimum over a batch of q points sampled jointly (propagate(full_cov=True) on the q points)."""
+
+    def __init__(self, y_min, d, q):
+        self.name = 'q-point Expected Improvement'
+        self.y_min = y_min
+        self.d = d
+        self.q = int(q)
+        self.IC_optimized = None
+        self.x_opt = None
+
+    def run(self, model, x, num_samples=1000, zs=None, seed=None, out=None):
+        """Returns -q-EI [G, D_L] of the G batches in x ([G q, d], batch g = rows g q .. g q + q - 1, or [G, q, d]). Batches are
+        independent of each other. One C-ABI call (dgp_qei); `out` is a result buffer to reuse, as in EI.run."""
+        if getattr(model, "name", None) != 'dgp':
+            raise NotImplementedError("only model.name == 'dgp' is on the accelerated path")
+        X = _lib.as_device(x, model.device)
+        if X.dim() == 3:
+            if X.shape[1] != self.q:
+                raise ValueError(f"x has shape {tuple(X.shape)}, expected [G, {self.q}, d]")
+            X = X.reshape(-1, X.shape[2])
+        X = model._check_X(X)
+        N, D = X.shape[0], model.layers[-1].num_outputs
+        own_out = out is None
+        if out is None:
+            out = torch.empty((N // self.q if self.q > 0 else 0, D), dtype=torch.float64, device=X.device)
+        if N == 0:
+            return out
+        m, keep = model._model_desc()
+        zt, zp = model._zs(zs, num_samples, N)
+        ctx = _lib.get_context(X.device)
+        ctx.call("dgp_qei", C.byref(m), _lib.ptr(X), N, num_samples, self.q, zp, model._next_seed(seed), 0, _scalar(self.y_min),
+                 _lib.ptr(out))
+        if own_out:
+            ctx.check()
+        return out
+
+    def optimize(self, model, bounds, popsize_DE=300, popstd_DE=1.5, iterations_DE=400, method='DE', num_samples=1000, seed=None):
+        """Minimise -q-EI over batches of q points in the box `bounds = (lw, up)`: differential evolution in q d dimensions (the box
+        tiled q times; member k decodes to the batch x[k].reshape(q, d)), one dgp_qei call per generation with fresh draws. Sets
+        and returns x_opt [q, d] (numpy); IC_optimized [1, D_L] is the criterion there. The full-covariance path has no adjoint,
+        so there is no Adam stage."""
+        if method in ('Adam', 'DE+Adam'):
+            raise NotImplementedError("q-EI has no input gradient (the full-covariance path has no adjoint): use method='DE'")
+        if method != 'DE':
+            raise ValueError(f"unknown method {method!r}")
+        if getattr(model, "name", None) != 'dgp':
+            raise NotImplementedError("only model.name == 'dgp' is on the accelerated path")
+        lw = np.broadcast_to(np.asarray(bounds[0], dtype=np.float64).reshape(-1), (self.d,))
+        up = np.broadcast_to(np.asarray(bounds[1], dtype=np.float64).reshape(-1), (self.d,))
+        qd = self.q * self.d
+        res = search.de_minimize(lambda X, out: self.run(model, X.reshape(-1, self.d), num_samples, out=out), np.tile(lw, self.q),
+                                 np.tile(up, self.q), qd, model.device, popsize_DE, popstd_DE, iterations_DE, seed=model._next_seed(seed))
+        self.x_opt = res["x"].cpu().numpy().reshape(self.q, self.d)
+        self.de_iterations = res["iterations"]
+        self.IC_optimized = self.run(model, self.x_opt, num_samples)
+        return self.x_opt
+
+
 def _scalar(v):
     return float(v.item() if hasattr(v, "item") else v)
 

@@ -9,7 +9,7 @@ from .gpflow_shim import RBF, Gaussian, Identity, Linear, Matern32, Matern52, Pa
 from .models.dgp import DGP, DGP_Base  # noqa: F401
 from .utils.layers import Layer, SVGP_Layer  # noqa: F401
 from .utils.layer_initializations import init_layers_linear  # noqa: F401
-from .Infill_criteria import EI, EV, WB2, WB2S, EV_one_constraint, PoF  # noqa: F401
+from .Infill_criteria import EI, EV, WB2, WB2S, EV_one_constraint, PoF, qEI  # noqa: F401
 from .EHVI import EHVI, EHVI_with_grad, EI_and_EHVI, HV_calcul, NDC, Y_ND, optimize_EHVI, psi  # noqa: F401
 from . import composite  # noqa: F401  (composite kernels with active_dims, layers on supplied kernel matrices: SURVEY §8 f2)
 from .models import MF_DGP  # noqa: F401

@@ -112,6 +112,9 @@ _SIG = {
                                          C.POINTER(_vp), C.POINTER(_vp)]),
     "dgp_propagate_full_cov_snd": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, C.POINTER(_vp),
                                              C.POINTER(_vp), C.POINTER(_vp)]),
+    "dgp_propagate_grouped_cov": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, _i, C.POINTER(_vp), _u64, _i64,
+                                            C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
+    "dgp_qei": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, _i, C.POINTER(_vp), _u64, _i64, _d, _vp]),
     "dgp_e_log_p_y": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, _vp]),
     "dgp_predict_moments": (C.c_int, [_vp, C.POINTER(ModelDesc), _vp, _i64, _i64, C.POINTER(_vp), _u64, _i64, _i,
                                       _vp, _vp]),

@@ -17,6 +17,7 @@
 #include "fused.cuh"
 #include "fused_bwd.cuh"
 #include "fullcov.cuh"
+#include "groupcov.cuh"
 #include "extk.cuh"
 #include "compkern.cuh"
 #include "gemm.cuh"
@@ -1864,6 +1865,129 @@ int dgp_propagate_full_cov_snd(dgp_ctx* c, const dgp_model_desc* model, const do
   CK(cudaSetDevice(c->device));
   RC(planned(c, [&] { return run_full_cov(c, model, X, true, N, S, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fvars_host); }));
   return check_chol(c);
+}
+
+namespace {
+// Grouped full_cov=True (groupcov.cuh): group g = points g q .. g q + q - 1 gets what run_full_cov gives for those q points alone
+// with n_offset + g q. The conditional (stash on) runs as in run_full_cov, then one grouped_cov_kernel per layer replaces the dense
+// blocks, their factorisation and the sample. Whole groups are processed in chunks sized to keep the arena under the workspace
+// limit; every output is per group, so the chunking does not change any value. qei_out: -q-EI [G][D_L] of the last layer's samples.
+int run_grouped_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, long N, long S, int q,
+                    const double* const* zs_host, unsigned long long seed, long n_offset, double* const* Fs_host,
+                    double* const* Fmeans_host, double* const* Fcovs_host, double* qei_out, double y_min) {
+  if (q < 1 || q > 32) { c->err = "grouped full_cov: the group size q must be in 1 .. 32"; return DGP_ERR_ARG; }
+  RC(check_chain(c, model, N, S));
+  if (N % q) { c->err = "grouped full_cov: N must be a multiple of the group size q"; return DGP_ERR_ARG; }
+  const int nl = model->num_layers;
+  const long G = N / q;
+  std::vector<LayerWs> lw;
+  RC(prep_layers(c, model, lw, PREP_FWD, {c->use_fused, true}));
+  int maxD = 1, maxMp = 0;
+  bool any_unfused = false;
+  size_t pp_doubles = 0;   // workspace doubles per padded point-sample
+  for (int l = 0; l < nl; ++l) {
+    const LayerWs& w = lw[l];
+    if (!moments_fit(c, w)) return DGP_ERR_UNSUPPORTED;
+    if (w.fcfg < 0) any_unfused = true;
+    if (w.D_out > maxD) maxD = w.D_out;
+    if (w.Mp > maxMp) maxMp = w.Mp;
+    pp_doubles += 4 * (size_t)w.D_out;                              // F, Fmean, Fvar, z
+  }
+  pp_doubles += (size_t)(1 + maxD) * maxMp;                          // V and T_d planes
+  if (any_unfused) pp_doubles += 2 * (size_t)maxMp;                  // Kuf, V of the unfused pipeline
+  long Gc_max;
+  {
+    const size_t fixed = c->used + ((size_t)8 << 20);
+    const size_t avail = c->ws_limit > fixed ? c->ws_limit - fixed : 0;
+    long pmax = (long)(avail / (pp_doubles * sizeof(double)));
+    pmax = pmax / kTileP * kTileP - kTileP;
+    Gc_max = pmax / (S * q);
+    if (Gc_max < 1) Gc_max = 1;
+    if (Gc_max > G) Gc_max = G;
+    const long nchunks = (G + Gc_max - 1) / Gc_max;   // equalise the chunks
+    Gc_max = (G + nchunks - 1) / nchunks;
+  }
+  const long Ppmax = round_up(Gc_max * q * S, kTileP);
+  std::vector<ChunkLayer> cls(nl);
+  for (int l = 0; l < nl; ++l) {
+    const LayerWs& w = lw[l];
+    cls[l].F = walloc(c, (size_t)Ppmax * w.D_out); cls[l].Fmean = walloc(c, (size_t)Ppmax * w.D_out);
+    cls[l].Fvar = walloc(c, (size_t)Ppmax * w.D_out); cls[l].z = walloc(c, (size_t)Ppmax * w.D_out);
+  }
+  double* planeV = walloc(c, (size_t)maxMp * Ppmax);
+  double* planeT = walloc(c, (size_t)maxD * maxMp * Ppmax);
+  Temps tmp;   // unfused layers: Kuf in t0, V in t1 (A goes to planeV)
+  if (any_unfused) { tmp.t0 = walloc(c, (size_t)maxMp * Ppmax); tmp.t1 = walloc(c, (size_t)maxMp * Ppmax); }
+  if (c->dry) return DGP_OK;
+
+  for (long g0 = 0; g0 < G; g0 += Gc_max) {
+    const long Gc = G - g0 < Gc_max ? G - g0 : Gc_max;
+    const long Nc = Gc * q, n0 = g0 * q, P = Nc * S, Pp = round_up(P, kTileP);
+    for (int l = 0; l < nl; ++l) {
+      const dgp_layer_desc& d = model->layers[l];
+      const LayerWs& w = lw[l];
+      ChunkLayer& cl = cls[l];
+      if (l == 0) { cl.Xin = X + n0 * d.D_in; cl.xmod = Nc; } else { cl.Xin = cls[l - 1].F; cl.xmod = P; }
+      cl.A = planeV; cl.T = planeT;
+      ChunkIO io;   // means go straight to the caller
+      std::vector<double*> fm(nl, nullptr);
+      if (Fmeans_host && Fmeans_host[l]) { fm[l] = Fmeans_host[l]; io.Fmeans = fm.data(); }
+      RC(forward_layer(c, d, w, cl, tmp, true, nullptr, l, Nc, S, N, n0, seed, n_offset, io, false));
+      CAT(DGP_CAT_MOMENTS);
+      const bool last = l == nl - 1;
+      const bool want_sample = !last || (Fs_host && Fs_host[l]) || qei_out;
+      GroupCovArgs a;
+      memset(&a, 0, sizeof(a));
+      a.V = w.fcfg >= 0 ? cl.A : tmp.t1; a.T = cl.T; a.Xin = cl.Xin; a.xmod = cl.xmod; a.D_in = w.D_in; a.ls = d.lengthscales;
+      a.var = d.variance; a.kind = d.kernel_kind; a.Mp = w.Mp; a.D = w.D_out; a.q = q; a.Nc = Nc; a.Pp = Pp; a.G = Gc; a.S = (int)S;
+      a.jitter = d.jitter; a.mean = cl.Fmean; a.F = cl.F; a.info = c->d_info;
+      a.F_user = (Fs_host && Fs_host[l]) ? Fs_host[l] : nullptr; a.N_total = N; a.n0 = n0;
+      a.cov_user = (Fcovs_host && Fcovs_host[l]) ? Fcovs_host[l] : nullptr; a.G_total = G; a.g0 = g0;
+      if (want_sample) {
+        if (zs_host && zs_host[l]) { a.z = zs_host[l] + n0 * w.D_out; a.z_ld = N; }
+        else {
+          const long total = P * w.D_out;
+          LAUNCH(philox_normal_kernel, (unsigned)((total + 255) / 256), 256, 0, seed, l, S, Nc, w.D_out, n_offset + n0, cl.z);
+          a.z = cl.z; a.z_ld = Nc;
+        }
+      }
+      const int qw = q <= 4 ? 4 : q <= 8 ? 8 : q <= 16 ? 16 : 32;
+      const unsigned grid = (unsigned)((Gc * S + kGcThreads / qw - 1) / (kGcThreads / qw));
+      switch (qw) {
+        case 4: LAUNCH(grouped_cov_kernel<4>, grid, kGcThreads, 0, a); break;
+        case 8: LAUNCH(grouped_cov_kernel<8>, grid, kGcThreads, 0, a); break;
+        case 16: LAUNCH(grouped_cov_kernel<16>, grid, kGcThreads, 0, a); break;
+        default: LAUNCH(grouped_cov_kernel<32>, grid, kGcThreads, 0, a); break;
+      }
+    }
+    if (qei_out) {
+      CAT(DGP_CAT_OTHER);
+      const int DL = lw[nl - 1].D_out;
+      const long warps = Gc * DL;
+      LAUNCH(qei_reduce_kernel, (unsigned)((warps * 32 + 127) / 128), 128, 0, cls[nl - 1].F, S, Nc, q, Gc, DL, y_min, qei_out + g0 * DL);
+    }
+  }
+  return DGP_OK;
+}
+}  // namespace
+
+int dgp_propagate_grouped_cov(dgp_ctx* c, const dgp_model_desc* model, const double* X, int64_t N, int64_t S, int q,
+                              const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
+                              double* const* Fmeans_host, double* const* Fcovs_host) {
+  if (!c || !model || !X) return DGP_ERR_ARG;
+  CK(cudaSetDevice(c->device));
+  RC(planned(c, [&] {
+    return run_grouped_cov(c, model, X, N, S, q, zs_host, seed, n_offset, Fs_host, Fmeans_host, Fcovs_host, nullptr, 0.0);
+  }));
+  return check_chol(c, "grouped full_cov: Kuu + jitter I or a q x q block + jitter I is not positive definite (Cholesky pivot <= 0)");
+}
+
+int dgp_qei(dgp_ctx* c, const dgp_model_desc* model, const double* X, int64_t N, int64_t S, int q, const double* const* zs_host,
+            uint64_t seed, int64_t n_offset, double y_min, double* out) {
+  if (!c || !model || !X) return DGP_ERR_ARG;
+  if (!out) { c->err = "dgp_qei: out is null"; return DGP_ERR_ARG; }
+  CK(cudaSetDevice(c->device));
+  return planned(c, [&] { return run_grouped_cov(c, model, X, N, S, q, zs_host, seed, n_offset, nullptr, nullptr, nullptr, out, y_min); });
 }
 
 namespace {

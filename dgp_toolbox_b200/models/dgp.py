@@ -87,27 +87,47 @@ class DGP_Base(_Module):
         return ts, _lib.ptr_array(ts)
 
     # ------------------------------------------------------------------ a7: propagate
-    def propagate(self, X, full_cov=False, S=1, zs=None, seed=None, n_offset=0):
+    def propagate(self, X, full_cov=False, S=1, zs=None, seed=None, n_offset=0, group_size=None):
         """dgp.py:34-63 -> (Fs, Fmeans, Fvars), lists of [S,N,D_l] tensors; full_cov=True draws samples correlated over the inputs
-        (Fvars then [S,N,N,D_l]: utils/layers.py:76-80,264-268; utils/utils.py:43-52)."""
+        (Fvars then [S,N,N,D_l]: utils/layers.py:76-80,264-268; utils/utils.py:43-52). With full_cov=True and group_size=q the
+        N points are N/q independent groups of q consecutive points: samples are correlated within a group only, group g is what
+        propagate(X[g q:(g+1) q], full_cov=True, n_offset=n_offset + g q) gives with the same seed, and Fvars[l] is
+        [S, N/q, q, q, D_l] (dgp_propagate_grouped_cov: 1 <= q <= 32, no limit on N)."""
+        if group_size is not None and not full_cov:
+            raise ValueError("group_size needs full_cov=True")
         X = self._check_X(_lib.as_device(X, self.device))
         N = X.shape[0]
         mk = lambda: [torch.empty((S, N, l.num_outputs), dtype=torch.float64, device=X.device) for l in self.layers]
         Fs, Fmeans = mk(), mk()
-        Fvars = [torch.empty((S, N, N, l.num_outputs), dtype=torch.float64, device=X.device) for l in self.layers] if full_cov else mk()
+        if group_size is not None:
+            q = int(group_size)
+            qs = max(q, 0)
+            G = N // q if q > 0 else 0
+            Fvars = [torch.empty((S, G, qs, qs, l.num_outputs), dtype=torch.float64, device=X.device) for l in self.layers]
+        elif full_cov:
+            Fvars = [torch.empty((S, N, N, l.num_outputs), dtype=torch.float64, device=X.device) for l in self.layers]
+        else:
+            Fvars = mk()
         if N == 0 or S == 0:
             return Fs, Fmeans, Fvars
         m, keep = self._model_desc()
         zt, zp = self._zs(zs, S, N)
-        _lib.get_context(X.device).call("dgp_propagate_full_cov" if full_cov else "dgp_propagate", C.byref(m), _lib.ptr(X), N, S, zp,
-                                        self._next_seed(seed), int(n_offset), _lib.ptr_array(Fs), _lib.ptr_array(Fmeans),
-                                        _lib.ptr_array(Fvars))
+        ctx = _lib.get_context(X.device)
+        if group_size is not None:
+            ctx.call("dgp_propagate_grouped_cov", C.byref(m), _lib.ptr(X), N, S, q, zp, self._next_seed(seed), int(n_offset),
+                     _lib.ptr_array(Fs), _lib.ptr_array(Fmeans), _lib.ptr_array(Fvars))
+            return Fs, Fmeans, Fvars
+        ctx.call("dgp_propagate_full_cov" if full_cov else "dgp_propagate", C.byref(m), _lib.ptr(X), N, S, zp,
+                 self._next_seed(seed), int(n_offset), _lib.ptr_array(Fs), _lib.ptr_array(Fmeans), _lib.ptr_array(Fvars))
         return Fs, Fmeans, Fvars
 
-    def predict_f(self, X, full_cov=False, S=1, zs=None, seed=None):
-        """dgp.py:66-77: last layer's mean [S,N,D_L] and variance [S,N,D_L] (full_cov=True: covariance [S,N,N,D_L])."""
+    def predict_f(self, X, full_cov=False, S=1, zs=None, seed=None, group_size=None):
+        """dgp.py:66-77: last layer's mean [S,N,D_L] and variance [S,N,D_L] (full_cov=True: covariance [S,N,N,D_L]; with
+        group_size=q, the [S,N/q,q,q,D_L] blocks of propagate(group_size=q))."""
+        if group_size is not None and not full_cov:
+            raise ValueError("group_size needs full_cov=True")
         if full_cov:
-            _, Fmeans, Fvars = self.propagate(X, full_cov=True, S=S, zs=zs, seed=seed)
+            _, Fmeans, Fvars = self.propagate(X, full_cov=True, S=S, zs=zs, seed=seed, group_size=group_size)
             return Fmeans[-1], Fvars[-1]
         X = self._check_X(_lib.as_device(X, self.device))
         N, L = X.shape[0], len(self.layers)

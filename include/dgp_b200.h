@@ -342,6 +342,21 @@ int dgp_propagate_full_cov_snd(dgp_ctx* ctx, const dgp_model_desc* model, const 
                                const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
                                double* const* Fmeans_host, double* const* Fvars_host);
 
+/* Grouped full_cov=True (batch acquisition): the N = G q points form G groups of q consecutive points, 1 <= q <= 32. Group g gets
+ * what dgp_propagate_full_cov gives for X[g q : (g + 1) q] alone with n_offset + g q and the same seed: samples correlated within
+ * the group, independent across groups. zs[l] [S, N, D_l] as dgp_propagate (group g uses columns g q ..). Caller arrays (any may
+ * be NULL): Fs[l], Fmeans[l] [S, N, D_l]; Fcovs[l] [S, G, q, q, D_l]. No limit on N: whole groups run in chunks sized to the
+ * workspace limit, with identical results. Refused before any launch: q outside 1 .. 32, N not a multiple of q. Forward only. */
+int dgp_propagate_grouped_cov(dgp_ctx* ctx, const dgp_model_desc* model, const double* X, int64_t N, int64_t S, int q,
+                              const double* const* zs_host, uint64_t seed, int64_t n_offset, double* const* Fs_host,
+                              double* const* Fmeans_host, double* const* Fcovs_host);
+
+/* Monte-Carlo q-EI of each group of dgp_propagate_grouped_cov: out [G, D_L] = -(1/S) sum_s max(y_min - min_j F_{s, g q + j}, 0)
+ * on the last layer's jointly drawn samples (the sign convention of dgp_ei). The sum over s runs in a fixed order. Does not
+ * synchronise (dgp_check reports a failed factorisation). */
+int dgp_qei(dgp_ctx* ctx, const dgp_model_desc* model, const double* X, int64_t N, int64_t S, int q,
+            const double* const* zs_host, uint64_t seed, int64_t n_offset, double y_min, double* out);
+
 /* DGP_Base.E_log_p_Y (models/dgp.py:79-87): out [N, D_L] = mean over the S samples of the Gaussian variational expectations
  * (-0.5 log 2pi - 0.5 log s_n^2 - 0.5 ((Y - mu)^2 + var) / s_n^2, utils/utils.py:89-93) of the last layer's moments. */
 int dgp_e_log_p_y(dgp_ctx* ctx, const dgp_model_desc* model, const double* X, const double* Y, int64_t N, int64_t S,
