@@ -82,9 +82,9 @@ def _mo_ehvi_with_grad(model_Y, Xcand, YND, S):
     N = X.shape[0]
     _, Fmeans, Fvars = m.propagate(X, S=S)
     mom = []
-    for o in (-2, -1):     # EHVI.py:126-130
-        mu = Fmeans[o].mean(0).reshape(-1)
-        mom += [mu, (Fvars[o] + Fmeans[o] ** 2).mean(0).reshape(-1) - mu ** 2]
+    for o in (-2, -1):     # EHVI.py:126-130, with the centred variance of dgp_mixture_moments (no cancellation at large |mean|)
+        mu = Fmeans[o].mean(0)
+        mom += [mu.reshape(-1), (Fvars[o].mean(0) + ((Fmeans[o] - mu) ** 2).mean(0)).reshape(-1)]
     val = torch.empty((N, 1), dtype=torch.float64, device=dev)
     g = torch.empty((N, 4), dtype=torch.float64, device=dev)
     y0 = _lib.as_device(np.asarray(YND[0], dtype=np.float64).reshape(-1), dev)

@@ -9,22 +9,25 @@ namespace dgp {
 __device__ __forceinline__ double norm_cdf(double x) { return 0.5 * erfc(-x * 0.70710678118654752440); }
 __device__ __forceinline__ double norm_pdf(double x) { return 0.39894228040143267794 * exp(-0.5 * x * x); }
 
-// mean[n,d] = mean_s mu ; var[n,d] = mean_s (v + add + mu^2) - mean^2     (inputs [S,N,D])
+// mean[n,d] = mean_s mu ; var[n,d] = mean_s (v + add) + mean_s (mu - mean)^2     (inputs [S,N,D])
+// Centred second pass: the one-pass mean_s (v + mu^2) - mean^2 cancels when |mean| is large next to the spread and can come out
+// zero or negative (then EI is NaN); this form has no cancellation and its error stays below S eps var.
 __global__ void mixture_moments_kernel(const double* __restrict__ Fmean, const double* __restrict__ Fvar, long S, long ND,
                                        const double* __restrict__ likvar, int add_lik, double* __restrict__ mean,
                                        double* __restrict__ var) {
   long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= ND) return;
   const double add = add_lik ? likvar[0] : 0.0;
-  double sm = 0.0, sq = 0.0;
+  double sm = 0.0;
+  for (long s = 0; s < S; ++s) sm += Fmean[s * ND + i];
+  const double mu = sm / (double)S;
+  double acc = 0.0;
   for (long s = 0; s < S; ++s) {
-    double m = Fmean[s * ND + i], v = Fvar[s * ND + i] + add;
-    sm += m;
-    sq += v + m * m;
+    const double d = Fmean[s * ND + i] - mu;
+    acc += (Fvar[s * ND + i] + add) + d * d;
   }
-  double mu = sm / (double)S;
   mean[i] = mu;
-  var[i] = sq / (double)S - mu * mu;
+  var[i] = acc / (double)S;
 }
 
 // -EI from moments: Normal(mean, sqrt(var)); t1 = (y_min - mean) cdf(y_min); t2 = var * pdf(y_min)
@@ -40,8 +43,8 @@ __global__ void ei_analytic_kernel(const double* __restrict__ mean, const double
 }
 
 // -EI and its upstream adjoints w.r.t. the last layer's per-sample moments (for d(-EI)/dx, the gradient the reference's
-// Adam-on-x acquisition search differentiates, Infill_criteria.py:79-84). With mbar = mean_s mu, vbar = mean_s(v + mu^2) - mbar^2,
-// sigma = sqrt(vbar), u = (y_min - mbar)/sigma:  d(-EI)/d mbar = Phi(u),  d(-EI)/d vbar = -phi(u) / (2 sigma), hence
+// Adam-on-x acquisition search differentiates, Infill_criteria.py:79-84). With mbar = mean_s mu, vbar = mean_s v + mean_s (mu - mbar)^2
+// (centred, as in mixture_moments_kernel), sigma = sqrt(vbar), u = (y_min - mbar)/sigma:  d(-EI)/d mbar = Phi(u),  d(-EI)/d vbar = -phi(u) / (2 sigma), hence
 //   Gm[s] = Phi(u)/S - phi(u) (mu_s - mbar) / (sigma S),   Gv[s] = -phi(u) / (2 sigma S).
 // One thread per candidate point; chunk-local p = s * Nc + n. Gm / GvT / GmPad / gq must be zero-filled beforehand.
 // kind selects the criterion c(mbar, vbar) (and its partial derivatives) evaluated on the mixture moments; lik_var != null adds
@@ -60,13 +63,15 @@ __global__ void ei_upstream_kernel(const double* __restrict__ Fmean, const doubl
   const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= Nc) return;
   for (int d = 0; d < D; ++d) {
-    double sm = 0.0, sq = 0.0;
+    double sm = 0.0;
+    for (long s = 0; s < S; ++s) sm += Fmean[(s * Nc + n) * D + d];
+    const double mbar = sm / (double)S;
+    double acc = 0.0;
     for (long s = 0; s < S; ++s) {
-      const double m = Fmean[(s * Nc + n) * D + d], v = Fvar[(s * Nc + n) * D + d];
-      sm += m;
-      sq += v + m * m;
+      const double dm_s = Fmean[(s * Nc + n) * D + d] - mbar;
+      acc += Fvar[(s * Nc + n) * D + d] + dm_s * dm_s;
     }
-    const double mbar = sm / (double)S, vbar = sq / (double)S - mbar * mbar + (lik_var ? lik_var[0] : 0.0), sig = sqrt(vbar);
+    const double vbar = acc / (double)S + (lik_var ? lik_var[0] : 0.0), sig = sqrt(vbar);
     double val = 0.0, dm, dv;
     if (kind == 4) {   // adjoints supplied by the caller (neg_ei holds (dc/dmbar, dc/dvbar) per candidate and output, read only)
       dm = neg_ei[(n * D + d) * 2];

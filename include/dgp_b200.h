@@ -384,7 +384,7 @@ int dgp_acq_moments(dgp_ctx* ctx, int kind, const double* mean, const double* va
 int dgp_ev_mc(dgp_ctx* ctx, const double* F, int64_t S, int64_t ND, double zero_c, double* out);
 /* Moment matching over the S samples of a propagated layer (models/dgp.py:362-366; EHVI.py:112-119 and the `mo_dgp` branch
  * :124-130, whose two objectives come out of ONE chain): Fmean, Fvar [S, ND] (DEVICE) -> mean [ND] = mean_s Fmean,
- * var [ND] = mean_s (Fvar + lik + Fmean^2) - mean^2; lik_variance (DEVICE, [1]) may be NULL (predict_f moments). */
+ * var [ND] = mean_s (Fvar + lik) + mean_s (Fmean - mean)^2 (centred: no cancellation at large |mean|); lik_variance (DEVICE, [1]) may be NULL (predict_f moments). */
 int dgp_mixture_moments(dgp_ctx* ctx, const double* Fmean, const double* Fvar, int64_t S, int64_t ND, const double* lik_variance,
                         double* mean, double* var);
 
